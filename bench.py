@@ -19,14 +19,20 @@ tiles are all-gathered with NCCL on a side stream, double-buffered, inside the t
   shard_parity (N > 1) one view ray-sharded N ways == rank 0's unsharded render bit for bit; sharded training gradients
   strong       (N > 1) ONE 800x800 view split N ways (strong scaling), gather included
   extra        config4 (vanilla hierarchical 64 + 128, 800x800) and config5 (4096-ray DepthNet training step), at 1 and N GPUs
+
+--dump-outputs DIR saves what the last timed step computed (rank 0's view) as float32 .npy files, so that two builds can be
+compared output for output: the inputs depend only on the arguments.  Nothing is written into the source tree, which may be
+read-only: a library older than its sources is recompiled into a temporary directory.
 """
 
 from __future__ import annotations
 
 import argparse
+import atexit
 import glob
 import json
 import os
+import shutil
 import statistics
 import subprocess
 import sys
@@ -36,6 +42,7 @@ import time
 
 import torch
 
+sys.dont_write_bytecode = True   # no __pycache__ in the tree
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
@@ -47,6 +54,7 @@ NERF_FLOP_EXECUTED = 1_056_768           # feature_linear folded into views_line
 DEPTHNET_FLOP_PER_RAY = 6_660_608        # literal network (the folded inference form executes 1,309,184)
 COMPOSITE_BYTES_PER_RAY = 24 * S + 36    # SURVEY.md 8(d)
 REF_CHUNK = 32768                        # one reference chunk (nerf_utils.py:88, BASELINE.md 3)
+DUMP_RAYS = 16384                        # rays whose per-sample arrays --dump-outputs keeps (1.5 KB each; all 640,000 are 0.98 GB)
 
 
 def peaks():
@@ -448,6 +456,19 @@ def shard_parity(models, dev, world, rank):
     return res
 
 
+def dump_outputs(out_dir, tile, mean, z, raw, acc, depth, weights):
+    """The arrays ops.render_depthnet(tile=True) would return for the last timed step, under its names, as float32 .npy: the
+    per-ray maps of the whole view, and z / weights / raw for a fixed, seeded sample of DUMP_RAYS rays (43 MB in all)."""
+    import numpy as np
+
+    sel = torch.randperm(z.shape[0], generator=torch.Generator().manual_seed(0))[:DUMP_RAYS].sort().values.to(z.device)
+    arrays = {"rgb": tile[:, :3], "disp": tile[:, 3], "acc": acc, "depth": depth, "z_mean": mean, "z": z[sel], "weights": weights[sel],
+              "raw": raw[sel]}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy().astype(np.float32))
+
+
 # ------------------------------------------------------------------------------------------------- our arm
 def main():
     ap = argparse.ArgumentParser()
@@ -461,7 +482,10 @@ def main():
     ap.add_argument("--ref-rays", type=int, default=REF_CHUNK, help="rays per step of the CPU reference arm (one reference chunk)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip config4 / config5 / strong / eager-GPU baseline")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -474,14 +498,16 @@ def main():
 
     import torch.distributed as dist
 
-    import nerf_sampling_b200 as pkg
-    from nerf_sampling_b200 import _lib, ops
+    from nerf_sampling_b200 import _build, _lib, ops
     from nerf_sampling_b200.nerf_pytorch import nerf_utils
     from nerf_sampling_b200.packing import PREC_FAST, PREC_FP16, PREC_SPLIT
 
     if not torch.cuda.is_available():
         raise SystemExit("bench.py: no CUDA device -- the B200 path has no CPU fallback (use --impl reference for the CPU arm)")
-    pkg.build()
+    if _build.is_stale():
+        tmp = tempfile.mkdtemp(prefix="b200nerf_")
+        atexit.register(shutil.rmtree, tmp, True)
+        _build.LIB_PATH = _build.build(out_path=os.path.join(tmp, "libb200nerf.so"))
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
     if world > 1:
@@ -581,6 +607,8 @@ def main():
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
     ms_total = float(ms)
     value = world * n_rays * args.steps / (ms_total * 1e-3)
+    if args.dump_outputs and rank == 0:   # before the e2e passes below reuse the buffers
+        dump_outputs(args.dump_outputs, tiles[(total_steps - 1) & 1], mean, z, raw, acc, depth, weights)
 
     k_ms = [statistics.mean(m[j].elapsed_time(m[j + 1]) for m in marks) for j in range(4)]  # depthnet, place, mlp, composite
     pk = peaks()
