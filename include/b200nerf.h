@@ -303,6 +303,22 @@ int b200nerf_umma_selftest(const uint16_t* A, const uint16_t* B, float* D, int K
 int b200nerf_debug_sgemm(int M, int N, int K, const float* A, long sAm, long sAk, const float* B, long sBk, long sBn, float* C,
                          int ldc, int beta, const float* bias, int act, float slope, int force_fp32, void* stream);
 
+/* Diagnostics: the kernels b200nerf_depthnet_train_fwd / _bwd / _jac / _bwd_jac pick for this architecture, batch and parameter
+ * alignment, as a bitmask of the predicates they call.  Host code only (reads the pointer values of params, launches nothing);
+ * a negative value on bad arguments.
+ *   COLLAPSED       the branches run as weight-only recurrences (chain_fwd / chain_bwd / chain_du, 2-CTA clusters), else per layer
+ *   FUSED_CHAIN     cat_layers.1 .. n_cat-1 + head in one launch of the split-precision MLP kernel, else per-layer 3xTF32 products
+ *   SPLIT_CAT0      cat_layers.0 as four split-K problems (its bias and LeakyReLU move into the fused chain's loader)
+ *   SPLIT_BACKWARD  _jac / _bwd_jac run the split backward, else _bwd_jac runs the one-pass backward
+ *   TENSOR_PATH     the one-pass backward runs on the tensor-core products, else on the CUDA-core head kernels and mixed products */
+#define B200NERF_ROUTE_COLLAPSED 1
+#define B200NERF_ROUTE_FUSED_CHAIN 2
+#define B200NERF_ROUTE_SPLIT_CAT0 4
+#define B200NERF_ROUTE_SPLIT_BACKWARD 8
+#define B200NERF_ROUTE_TENSOR_PATH 16
+int b200nerf_debug_depthnet_train_route(const float* const* params, int n_branch, const int* hidden, int n_cat, const int* cat_hidden,
+                                        int n_rays);
+
 /* Diagnostics: CTA 0 of every grouped-GEMM launch writes %globaltimer stamps (ns) of its phases into dev_buf (16 int64):
  * [0] entry, [1] barriers + TMEM ready, [2] last MMA retired, [3] epilogue stored, [4+c] chunk c handed to the MMA warp. */
 void b200nerf_debug_set_tgemm_timeline(long long* dev_buf);

@@ -56,6 +56,7 @@ SIGNATURES = {
     "b200nerf_umma_selftest": (I, [P, P, P, I, I, P]),
     "b200nerf_debug_set_tgemm_timeline": (None, [P]),
     "b200nerf_debug_sgemm": (I, [I, I, I, P, C.c_long, C.c_long, P, C.c_long, C.c_long, P, I, I, P, I, F, I, P]),
+    "b200nerf_debug_depthnet_train_route": (I, [P, I, P, I, P, I]),
     "b200nerf_depthnet_train_ws_floats": (SZ, [I, I, P, I, P]),
     "b200nerf_depthnet_n_params": (I, [I, I]),
     "b200nerf_depthnet_train_fwd": (I, [P, I, P, I, P, P, P, I, F, F, F, P, P, P]),

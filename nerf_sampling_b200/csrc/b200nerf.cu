@@ -487,7 +487,9 @@ extern "C" int b200nerf_nerf_pack_fast(const float* const* t, int prec, void* h_
 constexpr int DEPTHNET_MAX_HIDDEN = 10;
 static int depthnet_check(const char* who, int n_hidden, int prec) {
   if (prec != B200NERF_PREC_SPLIT) return fail("%s: prec must be B200NERF_PREC_SPLIT (the depth feeds the 2^9 octave of the encoding)", who);
-  if (n_hidden < 0 || n_hidden > DEPTHNET_MAX_HIDDEN) return fail("%s: n_hidden=%d out of range (0..%d)", who, n_hidden, DEPTHNET_MAX_HIDDEN);
+  if (n_hidden < 0 || n_hidden > DEPTHNET_MAX_HIDDEN)
+    return fail("%s: n_hidden=%d out of range (0..%d): inference serves DepthNets of 1 to %d cat layers", who, n_hidden, DEPTHNET_MAX_HIDDEN,
+                DEPTHNET_MAX_HIDDEN + 1);
   return 0;
 }
 extern "C" size_t b200nerf_depthnet_wpack_bytes(int n_hidden, int prec) {
@@ -504,9 +506,10 @@ extern "C" size_t b200nerf_depthnet_aux_floats(int n_hidden) {
 
 extern "C" int b200nerf_depthnet_pack(const float* h_w0, const float* h_b0, const float* const* h_hidden, int n_hidden,
                                       const float* h_head_w, const float* h_head_b, int prec, void* h_wpack, float* h_aux) {
+  // the architecture first: b200nerf_depthnet_wpack_bytes() is 0 for one it cannot serve, and a caller's empty buffer has no address
+  if (depthnet_check("b200nerf_depthnet_pack", n_hidden, prec)) return 1;
   if (!h_w0 || !h_b0 || !h_head_w || !h_head_b || !h_wpack || !h_aux || (n_hidden > 0 && !h_hidden))
     return fail("b200nerf_depthnet_pack: null argument");
-  if (depthnet_check("b200nerf_depthnet_pack", n_hidden, prec)) return 1;
   const int rc = pack_xprogram(depthnet_xprogram(h_w0, h_hidden, n_hidden), static_cast<uint8_t*>(h_wpack));
   if (rc) return rc;
   memset(h_aux, 0, b200nerf_depthnet_aux_floats(n_hidden) * sizeof(float));

@@ -899,6 +899,12 @@ static bool fused_chain_ok(const DnArch& ar, int n, const float* const* params) 
     if (reinterpret_cast<uintptr_t>(params[pidx_cat(ar, j)]) & 15) return false;
   return true;
 }
+// The split form of cat_layers.0 pays where the step is a latency chain (512 rays: 58 -> 26 us, step 0.60 -> 0.56 ms); at 4096 rays its
+// extra CTAs, atomics and memset cost SM time beside the target render (1.365 -> 1.41 ms).  It hands the bias and the LeakyReLU to the
+// fused chain's loader, so it needs that chain.
+static bool split_cat0(const DnArch& ar, int n, const float* const* params) { return fused_chain_ok(ar, n, params) && n <= 2048; }
+// Below 32 rays (or with B200NERF_TRAIN_GEMM=fp32) every pass runs per layer: CUDA-core head kernels and sgemm's product mix.
+static bool tensor_path_ok(int n) { return tgemm_enabled() && n >= 32; }
 static int chain_configure() {
   static bool configured[B200_MAX_DEVICES] = {false};
   const int dev = b200_device();
@@ -980,7 +986,7 @@ extern "C" int b200nerf_depthnet_train_fwd(const float* const* params, int n_bra
   depthnet_encode_kernel<<<(12 * n + 191) / 192, 192, 0, st>>>(rays_o, rays_d, n, radius, E);
   LAUNCH_CHECK();
   const int ed[3] = {63, 63, 126}, eo[3] = {0, 63, 126};
-  if (tgemm_enabled() && n >= 32) {
+  if (tensor_path_ok(n)) {
     const bool collapse = can_collapse(ar, n, params);
     if (collapse) {
       // collapsed branches: [A_i | c_i] recurrences over the weights (one launch), then x_last = e A_last^T + c_last per ray
@@ -1014,9 +1020,7 @@ extern "C" int b200nerf_depthnet_train_fwd(const float* const* params, int n_bra
     }
     const int hl = ar.h[ar.nb - 1];
     const bool fused = fused_chain_ok(ar, n, params);
-    // the split form of cat_layers.0 pays where the step is a latency chain (512 rays: 58 -> 26 us, step 0.60 -> 0.56 ms); at 4096
-    // rays its extra CTAs, atomics and memset cost SM time beside the target render (1.365 -> 1.41 ms)
-    const bool split0 = fused && n <= 2048;
+    const bool split0 = split_cat0(ar, n, params);
     {
       const float* W = params[pidx_cat(ar, 0)];
       const int ldw = 3 * hl + 252;
@@ -1190,7 +1194,7 @@ extern "C" int b200nerf_depthnet_train_bwd(const float* const* params, int n_bra
   // head: t = a_last . w + b, s = sigmoid(t), z = near + (far - near) s
   float* dt = ws + w.t;  // t itself is no longer needed
   const int ph = pidx_head(ar);
-  const bool tensor_path = tgemm_enabled() && n >= 32;
+  const bool tensor_path = tensor_path_ok(n);
   if (!tensor_path) {
     depth_head_bwd_kernel<<<(n + 255) / 256, 256, 0, st>>>(dz, ws + w.s, n, near_, far_, dt);
     LAUNCH_CHECK();
@@ -1326,7 +1330,7 @@ extern "C" int b200nerf_depthnet_train_bwd(const float* const* params, int n_bra
 // the losses are INDEPENDENT products,  dW_j = sum_r (dz_r J_j[r, :])^T x_{j-1}[r, :],  db_j = sum_r dz_r J_j[r, :],  one grouped
 // launch with dz applied to the k (ray) index of the A operand in the loader (tgemm `kscale`), then the weight-only branch chain.
 static bool split_backward_ok(const DnArch& ar, int n, const float* const* params) {
-  return tgemm_enabled() && n >= 32 && can_collapse(ar, n, params);
+  return tensor_path_ok(n) && can_collapse(ar, n, params);
 }
 extern "C" int b200nerf_depthnet_train_jac(const float* const* params, int n_branch, const int* hidden, int n_cat, const int* cat_hidden,
                                            int n_rays, float near_, float far_, float* ws, float* const* grads, void* stream) {
@@ -1857,4 +1861,21 @@ extern "C" int b200nerf_debug_sgemm(int M, int N, int K, const float* A, long sA
   sgemm_kernel<<<grid, 256, 0, st>>>(M, N, K, A, sAm, sAk, B, sBk, sBn, C, ldc, beta, bias, act, slope);
   LAUNCH_CHECK();
   return 0;
+}
+
+/* Which kernels the DepthNet training passes pick for this architecture, batch and parameter alignment, from the same predicates the
+   passes call (pure host code: only the pointer VALUES are read, nothing is launched). */
+extern "C" int b200nerf_debug_depthnet_train_route(const float* const* params, int n_branch, const int* hidden, int n_cat,
+                                                   const int* cat_hidden, int n_rays) {
+  if (!params || n_rays < 0) return -b200_fail("b200nerf_debug_depthnet_train_route: bad arguments");
+  DnArch ar;
+  if (dn_arch(n_branch, hidden, n_cat, cat_hidden, &ar)) return -1;
+  for (int v : ar.h)
+    if (v < 1) return -b200_fail("b200nerf_debug_depthnet_train_route: branch width %d", v);
+  for (int v : ar.c)
+    if (v < 1) return -b200_fail("b200nerf_debug_depthnet_train_route: cat width %d", v);
+  const int n = n_rays;
+  return (can_collapse(ar, n, params) ? B200NERF_ROUTE_COLLAPSED : 0) | (fused_chain_ok(ar, n, params) ? B200NERF_ROUTE_FUSED_CHAIN : 0) |
+         (split_cat0(ar, n, params) ? B200NERF_ROUTE_SPLIT_CAT0 : 0) | (split_backward_ok(ar, n, params) ? B200NERF_ROUTE_SPLIT_BACKWARD : 0) |
+         (tensor_path_ok(n) ? B200NERF_ROUTE_TENSOR_PATH : 0);
 }

@@ -147,7 +147,8 @@ def kernel_input_layout(rays_o, rays_d, radius=2.0):
     return torch.cat([O.embed(rays_o, 10), z, O.embed(rays_d, 10), z, O.embed(hits[:, 0], 10), z, O.embed(hits[:, 1], 10), z], -1)
 
 
-@pytest.mark.parametrize("widths", [([256] * 10, [256] * 10), ([128] * 6, [128, 128, 128, 128, 256]), ([64] * 2, [96])])
+@pytest.mark.parametrize("widths", [([256] * 10, [256] * 10), ([128] * 6, [128, 128, 128, 128, 256]), ([64] * 2, [96]),
+                                    ([200, 136, 256], [256, 256]), ([512] * 2, [256] * 3)])
 def test_fold_depthnet_matches_literal_network(widths):
     """Folding the activation-free branches into the first dense layer is exact up to fp32 round-off."""
     from nerf_sampling_b200.packing import fold_depthnet
