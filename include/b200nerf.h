@@ -62,14 +62,20 @@ int b200nerf_nerf_pack(const float* const* h_tensors, int prec, void* h_wpack, f
 
 /* DepthNet (depth_nets/depth_net.py:10-169) in inference form.  Its three branches apply no activation
  * (depth_net.py:140,148,156 are no-ops), so branches + cat_layers[0] are one affine map of the encodings.
- * The host folds them (fp64) into `h_w0` [256,256] / `h_b0` [256] over the kernel's input layout
- *   cols   0.. 62 enc(o) | 64..126 enc(d) | 128..190 enc(hit_near) | 192..254 enc(hit_far)   (63,127,191,255 = 0)
+ * The host folds them (fp64) into `h_w0` [256,256] / `h_b0` [256] over the kernel's input layout, four 64-column blocks
+ *   cols   0.. 63 enc(o) | 64..127 enc(d) | 128..191 enc(hit_near) | 192..255 enc(hit_far)
+ * of which the first d3 = 3 (1 + 2 multires) columns hold the encoding and the rest are zero (multires 10: 63 of 64).
  * `h_hidden` = n_hidden pairs (weight [256,256], bias [256]) of the remaining cat_layers (LeakyReLU 0.01),
- * `h_head_w` [256] / `h_head_b` [1] = to_depth.  Narrower layers are zero-padded to 256 by the caller. */
+ * `h_head_w` [256] / `h_head_b` [1] = to_depth.  Narrower layers are zero-padded to 256 by the caller.
+ * b200nerf_depthnet_pack_multires serves multires 1..10 and records it in the aux block, so b200nerf_depthnet_fwd and the
+ * render entry points encode the rays at the image's own multires; b200nerf_depthnet_pack is the same with multires 10. */
 size_t b200nerf_depthnet_wpack_bytes(int n_hidden, int prec);
 size_t b200nerf_depthnet_aux_floats(int n_hidden);
 int b200nerf_depthnet_pack(const float* h_w0, const float* h_b0, const float* const* h_hidden, int n_hidden,
                            const float* h_head_w, const float* h_head_b, int prec, void* h_wpack, float* h_aux);
+int b200nerf_depthnet_pack_multires(const float* h_w0, const float* h_b0, const float* const* h_hidden, int n_hidden,
+                                    const float* h_head_w, const float* h_head_b, int multires, int prec, void* h_wpack,
+                                    float* h_aux);
 
 /* ---- operators ------------------------------------------------------------------------------------------ */
 
@@ -224,17 +230,27 @@ int b200nerf_argmax_gather(const float* weights, const float* z, const float* ra
  * `params` = device pointers of the state_dict tensors in order: origin_layers.{i}.{weight,bias} (n_branch layers of
  * widths hidden[]), direction_layers..., intersection_layers..., cat_layers.{2j}.{weight,bias} (n_cat layers of widths
  * cat_hidden[]), to_depth.0.{weight,bias}: b200nerf_depthnet_n_params() pointers.  `ws` holds
- * b200nerf_depthnet_train_ws_floats() floats and carries the activations from fwd to bwd.  out_z [n_rays]. */
+ * b200nerf_depthnet_train_ws_floats() floats and carries the activations from fwd to bwd.  out_z [n_rays].
+ * The functions without a `multires` argument serve DepthNet(multires=10); their _multires forms take the positional-encoding
+ * size (1..10: gamma(o), gamma(d) are d3 = 3 (1 + 2 multires) wide, gamma(hits) 2 d3), which must be the same in every call of a step. */
 size_t b200nerf_depthnet_train_ws_floats(int n_rays, int n_branch, const int* hidden, int n_cat, const int* cat_hidden);
+size_t b200nerf_depthnet_train_ws_floats_multires(int n_rays, int n_branch, const int* hidden, int n_cat, const int* cat_hidden,
+                                                 int multires);
 int b200nerf_depthnet_n_params(int n_branch, int n_cat);
 int b200nerf_depthnet_train_fwd(const float* const* params, int n_branch, const int* hidden, int n_cat, const int* cat_hidden,
                                 const float* rays_o, const float* rays_d, int n_rays, float radius, float near_, float far_,
                                 float* ws, float* out_z, void* stream);
+int b200nerf_depthnet_train_fwd_multires(const float* const* params, int n_branch, const int* hidden, int n_cat, const int* cat_hidden,
+                                         int multires, const float* rays_o, const float* rays_d, int n_rays, float radius, float near_,
+                                         float far_, float* ws, float* out_z, void* stream);
 /* Backward of the above: dz [n_rays] -> gradients of every parameter, written (not accumulated) to `grads` (same order
  * and shapes as `params`).  Consumes the activations in `ws`. */
 int b200nerf_depthnet_train_bwd(const float* const* params, int n_branch, const int* hidden, int n_cat, const int* cat_hidden,
                                 int n_rays, float near_, float far_, float* ws, const float* dz, float* const* grads,
                                 void* stream);
+int b200nerf_depthnet_train_bwd_multires(const float* const* params, int n_branch, const int* hidden, int n_cat, const int* cat_hidden,
+                                         int multires, int n_rays, float near_, float far_, float* ws, const float* dz,
+                                         float* const* grads, void* stream);
 
 /* The same backward split at the losses (Trainer.py:525-538: both losses reach DepthNet through ONE scalar per ray, dz, and the
  * backward is linear in it).  b200nerf_depthnet_train_jac runs BEFORE the losses exist: it zeroes `grads` and walks the sequential
@@ -250,6 +266,11 @@ int b200nerf_depthnet_train_jac(const float* const* params, int n_branch, const 
 int b200nerf_depthnet_train_bwd_jac(const float* const* params, int n_branch, const int* hidden, int n_cat, const int* cat_hidden,
                                     int n_rays, float near_, float far_, float* ws, const float* dz, float* const* grads,
                                     void* stream, void* stream_aux);
+int b200nerf_depthnet_train_jac_multires(const float* const* params, int n_branch, const int* hidden, int n_cat, const int* cat_hidden,
+                                         int multires, int n_rays, float near_, float far_, float* ws, float* const* grads, void* stream);
+int b200nerf_depthnet_train_bwd_jac_multires(const float* const* params, int n_branch, const int* hidden, int n_cat,
+                                             const int* cat_hidden, int multires, int n_rays, float near_, float far_, float* ws,
+                                             const float* dz, float* const* grads, void* stream, void* stream_aux);
 
 /* The frozen NeRF at ONE sample per ray, p = o + d z (nerf_utils.py:693-715), in fp32, together with d raw / d z
  * (forward-mode derivative along the ray: what loss.backward() propagates from the colour into DepthNet's depth).
@@ -318,6 +339,8 @@ int b200nerf_debug_sgemm(int M, int N, int K, const float* A, long sAm, long sAk
 #define B200NERF_ROUTE_TENSOR_PATH 16
 int b200nerf_debug_depthnet_train_route(const float* const* params, int n_branch, const int* hidden, int n_cat, const int* cat_hidden,
                                         int n_rays);
+int b200nerf_debug_depthnet_train_route_multires(const float* const* params, int n_branch, const int* hidden, int n_cat,
+                                                 const int* cat_hidden, int multires, int n_rays);
 
 /* Diagnostics: CTA 0 of every grouped-GEMM launch writes %globaltimer stamps (ns) of its phases into dev_buf (16 int64):
  * [0] entry, [1] barriers + TMEM ready, [2] last MMA retired, [3] epilogue stored, [4+c] chunk c handed to the MMA warp. */

@@ -29,6 +29,7 @@ SIGNATURES = {
     "b200nerf_depthnet_wpack_bytes": (SZ, [I, I]),
     "b200nerf_depthnet_aux_floats": (SZ, [I]),
     "b200nerf_depthnet_pack": (I, [P, P, P, I, P, P, I, P, P]),
+    "b200nerf_depthnet_pack_multires": (I, [P, P, P, I, P, P, I, I, P, P]),
     "b200nerf_get_rays": (I, [I, I, F, F, F, F, P, P, P, P, P]),
     "b200nerf_get_rays_at": (I, [I, I, F, F, F, F, P, P, I, P, P, P, P]),
     "b200nerf_gather_pixels": (I, [P, P, I, I, P, P]),
@@ -57,12 +58,18 @@ SIGNATURES = {
     "b200nerf_debug_set_tgemm_timeline": (None, [P]),
     "b200nerf_debug_sgemm": (I, [I, I, I, P, C.c_long, C.c_long, P, C.c_long, C.c_long, P, I, I, P, I, F, I, P]),
     "b200nerf_debug_depthnet_train_route": (I, [P, I, P, I, P, I]),
+    "b200nerf_debug_depthnet_train_route_multires": (I, [P, I, P, I, P, I, I]),
     "b200nerf_depthnet_train_ws_floats": (SZ, [I, I, P, I, P]),
+    "b200nerf_depthnet_train_ws_floats_multires": (SZ, [I, I, P, I, P, I]),
     "b200nerf_depthnet_n_params": (I, [I, I]),
     "b200nerf_depthnet_train_fwd": (I, [P, I, P, I, P, P, P, I, F, F, F, P, P, P]),
+    "b200nerf_depthnet_train_fwd_multires": (I, [P, I, P, I, P, I, P, P, I, F, F, F, P, P, P]),
     "b200nerf_depthnet_train_bwd": (I, [P, I, P, I, P, I, F, F, P, P, P, P]),
+    "b200nerf_depthnet_train_bwd_multires": (I, [P, I, P, I, P, I, I, F, F, P, P, P, P]),
     "b200nerf_depthnet_train_jac": (I, [P, I, P, I, P, I, F, F, P, P, P]),
+    "b200nerf_depthnet_train_jac_multires": (I, [P, I, P, I, P, I, I, F, F, P, P, P]),
     "b200nerf_depthnet_train_bwd_jac": (I, [P, I, P, I, P, I, F, F, P, P, P, P, P]),
+    "b200nerf_depthnet_train_bwd_jac_multires": (I, [P, I, P, I, P, I, I, F, F, P, P, P, P, P]),
     "b200nerf_nerf_point_ws_floats": (SZ, [I]),
     "b200nerf_nerf_point_jvp": (I, [P, P, P, P, P, I, P, P, P, P]),
     "b200nerf_nerf_point_jvp_packed_ws_bytes": (SZ, [I]),

@@ -504,10 +504,13 @@ extern "C" size_t b200nerf_depthnet_aux_floats(int n_hidden) {
   return need > static_cast<size_t>(exact::AUX_FLOATS) ? need : static_cast<size_t>(exact::AUX_FLOATS);
 }
 
-extern "C" int b200nerf_depthnet_pack(const float* h_w0, const float* h_b0, const float* const* h_hidden, int n_hidden,
-                                      const float* h_head_w, const float* h_head_b, int prec, void* h_wpack, float* h_aux) {
+extern "C" int b200nerf_depthnet_pack_multires(const float* h_w0, const float* h_b0, const float* const* h_hidden, int n_hidden,
+                                               const float* h_head_w, const float* h_head_b, int multires, int prec, void* h_wpack,
+                                               float* h_aux) {
   // the architecture first: b200nerf_depthnet_wpack_bytes() is 0 for one it cannot serve, and a caller's empty buffer has no address
   if (depthnet_check("b200nerf_depthnet_pack", n_hidden, prec)) return 1;
+  // enc(o) at multires 10 is 63 wide: every encoding fills at most the 64 columns of its block of the layer-0 operand
+  if (multires < 1 || multires > 10) return fail("b200nerf_depthnet_pack: multires=%d out of range (1..10)", multires);
   if (!h_w0 || !h_b0 || !h_head_w || !h_head_b || !h_wpack || !h_aux || (n_hidden > 0 && !h_hidden))
     return fail("b200nerf_depthnet_pack: null argument");
   const int rc = pack_xprogram(depthnet_xprogram(h_w0, h_hidden, n_hidden), static_cast<uint8_t*>(h_wpack));
@@ -518,8 +521,13 @@ extern "C" int b200nerf_depthnet_pack(const float* h_w0, const float* h_b0, cons
   memcpy(h_aux + 256 * (n_hidden + 1), h_head_w, 256 * sizeof(float));
   float* hb = h_aux + 256 * (n_hidden + 2);
   hb[0] = h_head_b[0];
-  hb[1] = hb[2] = hb[3] = 0.f;
+  hb[1] = multires == 10 ? 0.f : static_cast<float>(multires);   // the encoder's multires; 0 means 10 (images packed before it was stored)
+  hb[2] = hb[3] = 0.f;
   return 0;
+}
+extern "C" int b200nerf_depthnet_pack(const float* h_w0, const float* h_b0, const float* const* h_hidden, int n_hidden,
+                                      const float* h_head_w, const float* h_head_b, int prec, void* h_wpack, float* h_aux) {
+  return b200nerf_depthnet_pack_multires(h_w0, h_b0, h_hidden, n_hidden, h_head_w, h_head_b, 10, prec, h_wpack, h_aux);
 }
 
 // ------------------------------------------------------------------------------------------- ray generation

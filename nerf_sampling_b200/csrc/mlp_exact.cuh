@@ -229,6 +229,33 @@ __device__ __forceinline__ void encode_store_img(const float (&x)[3], uint8_t* d
   }
 }
 
+// DepthNet's input tile in the staging image: enc(o) | enc(d) | enc(hit_near) | enc(hit_far), 64 columns each (NF = multires;
+// columns 3 + 6 NF .. 63 of each block are zero)
+template <int NF>
+__device__ __forceinline__ void depthnet_encode_img(const float (&o)[3], const float (&d)[3], const float (&p0)[3], const float (&p1)[3],
+                                                    uint8_t* img) {
+  encode_store_img<NF, 8>(o, img, 32 * KC_STRIDE);
+  encode_store_img<NF, 8>(d, img + 8 * KC_STRIDE, 32 * KC_STRIDE);
+  encode_store_img<NF, 8>(p0, img + 16 * KC_STRIDE, 32 * KC_STRIDE);
+  encode_store_img<NF, 8>(p1, img + 24 * KC_STRIDE, 32 * KC_STRIDE);
+}
+
+// multires 1..9, out of line: their encoders stay out of the kernel's hot code
+__device__ __noinline__ void depthnet_encode_img_lt10(int nf, const float (&o)[3], const float (&d)[3], const float (&p0)[3],
+                                                      const float (&p1)[3], uint8_t* img) {
+  switch (nf) {
+    case 1: depthnet_encode_img<1>(o, d, p0, p1, img); break;
+    case 2: depthnet_encode_img<2>(o, d, p0, p1, img); break;
+    case 3: depthnet_encode_img<3>(o, d, p0, p1, img); break;
+    case 4: depthnet_encode_img<4>(o, d, p0, p1, img); break;
+    case 5: depthnet_encode_img<5>(o, d, p0, p1, img); break;
+    case 6: depthnet_encode_img<6>(o, d, p0, p1, img); break;
+    case 7: depthnet_encode_img<7>(o, d, p0, p1, img); break;
+    case 8: depthnet_encode_img<8>(o, d, p0, p1, img); break;
+    default: depthnet_encode_img<9>(o, d, p0, p1, img); break;
+  }
+}
+
 // eight consecutive floats as ONE 256-bit store (STG.E.256: a full 32-byte sector per lane and instruction; the rows of a tile are
 // 1 KB apart, so the lanes of a warp can never share a sector)
 __device__ __forceinline__ void st_global_v8(float* p, const float (&x)[8]) {
@@ -588,7 +615,7 @@ __global__ void __launch_bounds__(THREADS, 1) mlp_exact_kernel(const __grid_cons
         __syncwarp();
         if (lane == 0) mbar_arrive_remote(rv_bar);
       } else {
-        // DepthNet: 120 accurate sincosf per ray are far too slow to sit between two tiles, so the encoders work one
+        // DepthNet: 12 multires (120) accurate sincosf per ray are far too slow to sit between two tiles, so the encoders work one
         // tile AHEAD into a per-CTA staging image in global memory (L2-resident, already in the operand layout); when the
         // previous tile releases the operand columns, one lane pulls the image in with two bulk TMA copies per half.
         //   part 1 = enc(o) | enc(d) -> K chunks 0..15, part 2 = enc(hit_near) | enc(hit_far) -> K chunks 16..31
@@ -617,10 +644,11 @@ __global__ void __launch_bounds__(THREADS, 1) mlp_exact_kernel(const __grid_cons
           p0[t] = __fadd_rn(o[t], __fmul_rn(t0, d[t]));
           p1[t] = __fadd_rn(o[t], __fmul_rn(t1, d[t]));
         }
-        encode_store_img<10, 8>(o, stage_img + row_off, 32 * KC_STRIDE);
-        encode_store_img<10, 8>(d, stage_img + 8 * KC_STRIDE + row_off, 32 * KC_STRIDE);
-        encode_store_img<10, 8>(p0, stage_img + 16 * KC_STRIDE + row_off, 32 * KC_STRIDE);
-        encode_store_img<10, 8>(p1, stage_img + 24 * KC_STRIDE + row_off, 32 * KC_STRIDE);
+        // the image's multires sits in the aux slot after the head bias (0 = 10, the images packed before the slot was used);
+        // uniform over the CTA; multires 10 runs the fixed-10 encoder inline, the smaller sizes sit out of line
+        const int nf = static_cast<int>(saux[p.head_b_off + 1]);
+        if (nf == 0 || nf == 10) depthnet_encode_img<10>(o, d, p0, p1, stage_img + row_off);
+        else depthnet_encode_img_lt10(nf, o, d, p0, p1, stage_img + row_off);
         __threadfence();
         fence_proxy_async_all();                       // generic-proxy global writes -> visible to the bulk copy engine
         named_bar_sync(6, PRO_WARPS * 32);

@@ -321,11 +321,11 @@ static int colsum(cudaStream_t st, const float* dY, int n, int M, int ldy, float
 }
 
 // ------------------------------------------------------------------------------------------- encodings
-// gamma(x) of a C-vector: [x, sin(2^0 x), cos(2^0 x), ...] (run_nerf_helpers.py:15-63), C*(1+2F) wide
-// E[n, 252] = [gamma(o) 63 | gamma(d) 63 | gamma([hit_near, hit_far]) 126]; sphere hits in the reference's op order
+// gamma(x) of a C-vector: [x, sin(2^0 x), cos(2^0 x), ...] (run_nerf_helpers.py:15-63), C*(1+2F) wide, F = multires
+// E[n, 4 d3] = [gamma(o) d3 | gamma(d) d3 | gamma([hit_near, hit_far]) 2 d3], d3 = 3 (1 + 2F); sphere hits in the reference's op order
 // (nerf_pytorch/utils.py:159-217), NaN when the ray misses.  Twelve threads per ray -- (vector o / d / hit_near / hit_far) x channel --
-// so that a thread runs 10 accurate sincosf instead of 120 in a row (the kernel is latency-, not throughput-bound: 4096 rays).
-__global__ void depthnet_encode_kernel(const float* __restrict__ ro, const float* __restrict__ rd, int n, float radius,
+// so that a thread runs F accurate sincosf instead of 12 F in a row (the kernel is latency-, not throughput-bound: 4096 rays).
+__global__ void depthnet_encode_kernel(const float* __restrict__ ro, const float* __restrict__ rd, int n, float radius, int nf,
                                        float* __restrict__ E) {
   const int t = blockIdx.x * blockDim.x + threadIdx.x;
   const int i = t / 12, part = (t % 12) / 3, c = t % 3;
@@ -355,9 +355,10 @@ __global__ void depthnet_encode_kernel(const float* __restrict__ ro, const float
   // gamma of a C-vector is [x (C), sin(2^0 x) (C), cos(2^0 x) (C), ...]: o and d are 3-vectors, the two hit points one 6-vector
   const int C = part < 2 ? 3 : 6;
   const int ch = part < 2 ? c : (part - 2) * 3 + c;
-  float* e = E + static_cast<size_t>(i) * 252 + (part == 0 ? 0 : (part == 1 ? 63 : 126));
+  const int d3 = 3 * (1 + 2 * nf);
+  float* e = E + static_cast<size_t>(i) * (4 * d3) + (part == 0 ? 0 : (part == 1 ? d3 : 2 * d3));
   e[ch] = x;
-  for (int j = 0; j < 10; ++j) {
+  for (int j = 0; j < nf; ++j) {
     float sn, cs;
     sincosf(x * static_cast<float>(1 << j), &sn, &cs);
     e[C + j * 2 * C + ch] = sn;
@@ -461,7 +462,7 @@ struct ChainBranch {
   float* gW[CH_MAXL];
   float* gb[CH_MAXL];
   int h[CH_MAXL];
-  int d;              // encoding width (63 / 63 / 126)
+  int d;              // encoding width (d3 / d3 / 2 d3: 63 / 63 / 126 at multires 10)
   int cta_begin;      // first CTA of this branch in the launch
   float* Aaug;        // [L][CH_MAXH][CH_LD]: [A_i | c_i]
   float* Raug;        // [L][CH_MAXH][CH_LD]: R_i
@@ -816,6 +817,10 @@ struct DnArch {
   int nc;                 // cat layers
   std::vector<int> h;     // branch widths [nb]
   std::vector<int> c;     // cat widths [nc]
+  int m;                  // multires: gamma(o) / gamma(d) are d3 = 3 (1 + 2 m) wide, gamma(hits) 2 d3
+  int d3, ew;             // d3 and the row width of the encoding E, ew = 4 d3 (= the K of cat_layers.0's encoding segment)
+  int ed(int b) const { return b == 2 ? 2 * d3 : d3; }   // encoding width of branch b (origin / direction / intersection)
+  int eo(int b) const { return b * d3; }                 // its column offset in E
 };
 struct DnWs {             // float offsets into the workspace
   size_t E, s, t, total;
@@ -831,7 +836,7 @@ static DnWs dn_layout(const DnArch& ar, size_t n) {
   DnWs w;
   size_t o = 0;
   auto take = [&](size_t f) { size_t r = o; o += (f + 63) & ~static_cast<size_t>(63); return r; };
-  w.E = take(n * 252);
+  w.E = take(n * ar.ew);
   for (int b = 0; b < 3; ++b)
     for (int i = 0; i < ar.nb; ++i) w.xb[b].push_back(take(n * ar.h[i]));
   for (int j = 0; j < ar.nc; ++j) w.a.push_back(take(n * ar.c[j]));
@@ -862,12 +867,17 @@ static DnWs dn_layout(const DnArch& ar, size_t n) {
   w.total = o;
   return w;
 }
-static int dn_arch(int nb, const int* h, int nc, const int* c, DnArch* ar) {
+static int dn_arch(int nb, const int* h, int nc, const int* c, int multires, DnArch* ar) {
   if (nb < 1 || nc < 1 || !h || !c) return b200_fail("DepthNet architecture: bad arguments");
+  // multires 10 is the widest encoding the collapsed-branch chain matrices hold: 2 d3 + 1 = 127 columns of CH_LD
+  if (multires < 1 || multires > 10) return b200_fail("DepthNet architecture: multires=%d out of range (1..10)", multires);
   ar->nb = nb;
   ar->nc = nc;
   ar->h.assign(h, h + nb);
   ar->c.assign(c, c + nc);
+  ar->m = multires;
+  ar->d3 = 3 * (1 + 2 * multires);
+  ar->ew = 4 * ar->d3;
   return 0;
 }
 // parameter order = state_dict order: origin_layers.{i}.{w,b}, direction_layers..., intersection_layers...,
@@ -919,7 +929,7 @@ static int chain_configure() {
 static ChainParams chain_params(const DnArch& ar, const DnWs& w, float* ws, const float* const* params, float* const* grads) {
   ChainParams cp;
   memset(&cp, 0, sizeof(cp));
-  const int ed[3] = {63, 63, 126};
+  const int ed[3] = {ar.ed(0), ar.ed(1), ar.ed(2)};
   cp.L = ar.nb;
   int cta = 0;
   for (int b = 0; b < 3; ++b) {
@@ -965,27 +975,31 @@ static int launch_chain(void (*kern)(const ChainParams), const ChainParams& cp, 
   return 0;
 }
 
-extern "C" size_t b200nerf_depthnet_train_ws_floats(int n_rays, int n_branch, const int* hidden, int n_cat, const int* cat_hidden) {
+extern "C" size_t b200nerf_depthnet_train_ws_floats_multires(int n_rays, int n_branch, const int* hidden, int n_cat, const int* cat_hidden,
+                                                            int multires) {
   DnArch ar;
-  if (dn_arch(n_branch, hidden, n_cat, cat_hidden, &ar)) return 0;
+  if (dn_arch(n_branch, hidden, n_cat, cat_hidden, multires, &ar)) return 0;
   return dn_layout(ar, static_cast<size_t>(n_rays)).total;
+}
+extern "C" size_t b200nerf_depthnet_train_ws_floats(int n_rays, int n_branch, const int* hidden, int n_cat, const int* cat_hidden) {
+  return b200nerf_depthnet_train_ws_floats_multires(n_rays, n_branch, hidden, n_cat, cat_hidden, 10);
 }
 extern "C" int b200nerf_depthnet_n_params(int n_branch, int n_cat) { return (3 * n_branch + n_cat + 1) * 2; }
 
-extern "C" int b200nerf_depthnet_train_fwd(const float* const* params, int n_branch, const int* hidden, int n_cat,
-                                           const int* cat_hidden, const float* rays_o, const float* rays_d, int n_rays, float radius,
-                                           float near_, float far_, float* ws, float* out_z, void* stream) {
+extern "C" int b200nerf_depthnet_train_fwd_multires(const float* const* params, int n_branch, const int* hidden, int n_cat,
+                                                    const int* cat_hidden, int multires, const float* rays_o, const float* rays_d, int n_rays,
+                                                    float radius, float near_, float far_, float* ws, float* out_z, void* stream) {
   if (n_rays <= 0) return 0;
   if (!params || !rays_o || !rays_d || !ws || !out_z) return b200_fail("b200nerf_depthnet_train_fwd: null argument");
   DnArch ar;
-  if (dn_arch(n_branch, hidden, n_cat, cat_hidden, &ar)) return 1;
+  if (dn_arch(n_branch, hidden, n_cat, cat_hidden, multires, &ar)) return 1;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const int n = n_rays;
   const DnWs w = dn_layout(ar, n);
   float* E = ws + w.E;
-  depthnet_encode_kernel<<<(12 * n + 191) / 192, 192, 0, st>>>(rays_o, rays_d, n, radius, E);
+  depthnet_encode_kernel<<<(12 * n + 191) / 192, 192, 0, st>>>(rays_o, rays_d, n, radius, ar.m, E);
   LAUNCH_CHECK();
-  const int ed[3] = {63, 63, 126}, eo[3] = {0, 63, 126};
+  const int ed[3] = {ar.ed(0), ar.ed(1), ar.ed(2)}, eo[3] = {ar.eo(0), ar.eo(1), ar.eo(2)};
   if (tensor_path_ok(n)) {
     const bool collapse = can_collapse(ar, n, params);
     if (collapse) {
@@ -997,7 +1011,7 @@ extern "C" int b200nerf_depthnet_train_fwd(const float* const* params, int n_bra
       const int hlast = ar.h[ar.nb - 1];
       for (int b = 0; b < 3; ++b) {
         q[b] = prob_fwd(n, hlast, ws + w.xb[b][ar.nb - 1], hlast, ws + w.c_last[b], 0, 0.f);
-        seg_fwd(q[b], E + eo[b], 252, ws + w.Aaug[b] + static_cast<size_t>(ar.nb - 1) * CH_MAXH * CH_LD, CH_LD, 0, ed[b]);
+        seg_fwd(q[b], E + eo[b], ar.ew, ws + w.Aaug[b] + static_cast<size_t>(ar.nb - 1) * CH_MAXH * CH_LD, CH_LD, 0, ed[b]);
       }
       if (tgemm_group(st, q, 3)) return 1;
     }
@@ -1010,11 +1024,11 @@ extern "C" int b200nerf_depthnet_train_fwd(const float* const* params, int n_bra
         const float* W = params[pidx_branch(ar, b, i)];
         const int prev_w = i == 0 ? ed[b] : ar.h[i - 1];
         const float* prev = i == 0 ? e : ws + w.xb[b][i - 1];
-        const int prev_ld = i == 0 ? 252 : ar.h[i - 1];
+        const int prev_ld = i == 0 ? ar.ew : ar.h[i - 1];
         const int ldw = prev_w + ed[b];
         q[b] = prob_fwd(n, ar.h[i], ws + w.xb[b][i], ar.h[i], params[pidx_branch(ar, b, i) + 1], 0, 0.f);
         seg_fwd(q[b], prev, prev_ld, W, ldw, 0, prev_w);
-        seg_fwd(q[b], e, 252, W, ldw, prev_w, ed[b]);
+        seg_fwd(q[b], e, ar.ew, W, ldw, prev_w, ed[b]);
       }
       if (tgemm_group(st, q, 3)) return 1;
     }
@@ -1023,7 +1037,7 @@ extern "C" int b200nerf_depthnet_train_fwd(const float* const* params, int n_bra
     const bool split0 = split_cat0(ar, n, params);
     {
       const float* W = params[pidx_cat(ar, 0)];
-      const int ldw = 3 * hl + 252;
+      const int ldw = 3 * hl + ar.ew;
       if (split0) {
         // cat_layers.0 as FOUR split-K problems (one per K segment, two K slices each) that add into the zeroed output: K = 1020 in
         // one CTA is 32 chunks and, at 512 rays, the longest launch in front of the fused chain (58 us); the bias and the LeakyReLU
@@ -1035,7 +1049,7 @@ extern "C" int b200nerf_depthnet_train_fwd(const float* const* params, int n_bra
           seg_fwd(q[b], ws + w.xb[b][ar.nb - 1], hl, W, ldw, b * hl, hl);
         }
         q[3] = prob_fwd(n, ar.c[0], ws + w.a[0], ar.c[0], nullptr, 0, 0.f);
-        seg_fwd(q[3], E, 252, W, ldw, 3 * hl, 252);
+        seg_fwd(q[3], E, ar.ew, W, ldw, 3 * hl, ar.ew);
         for (int i = 0; i < 4; ++i) {
           q[i].force_splits = 2;
           q[i].c_zeroed = true;
@@ -1044,7 +1058,7 @@ extern "C" int b200nerf_depthnet_train_fwd(const float* const* params, int n_bra
       } else {
         GemmProb q = prob_fwd(n, ar.c[0], ws + w.a[0], ar.c[0], params[pidx_cat(ar, 0) + 1], 1, 0.01f);
         for (int b = 0; b < 3; ++b) seg_fwd(q, ws + w.xb[b][ar.nb - 1], hl, W, ldw, b * hl, hl);
-        seg_fwd(q, E, 252, W, ldw, 3 * hl, 252);
+        seg_fwd(q, E, ar.ew, W, ldw, 3 * hl, ar.ew);
         if (tgemm_group(st, &q, 1)) return 1;
       }
     }
@@ -1085,11 +1099,11 @@ extern "C" int b200nerf_depthnet_train_fwd(const float* const* params, int n_bra
       float* y = ws + w.xb[b][i];
       const int prev_w = i == 0 ? ed[b] : ar.h[i - 1];
       const float* prev = i == 0 ? e : ws + w.xb[b][i - 1];
-      const int prev_ld = i == 0 ? 252 : ar.h[i - 1];
+      const int prev_ld = i == 0 ? ar.ew : ar.h[i - 1];
       const int ldw = prev_w + ed[b];
       // x = Linear(cat([x_prev, e])) -- no activation (depth_net.py:140,148,156 construct a module and drop it)
       if (lin_fwd(st, n, ar.h[i], prev_w, prev, prev_ld, W, ldw, 0, y, ar.h[i], 0, nullptr, 0, 0.f)) return 1;
-      if (lin_fwd(st, n, ar.h[i], ed[b], e, 252, W, ldw, prev_w, y, ar.h[i], 1, bias, 0, 0.f)) return 1;
+      if (lin_fwd(st, n, ar.h[i], ed[b], e, ar.ew, W, ldw, prev_w, y, ar.h[i], 1, bias, 0, 0.f)) return 1;
     }
   }
   const int hl = ar.h[ar.nb - 1];
@@ -1097,11 +1111,11 @@ extern "C" int b200nerf_depthnet_train_fwd(const float* const* params, int n_bra
     // cat_layers.0 over cat([x_o, x_d, x_i, e_o, e_d, e_i])
     const float* W = params[pidx_cat(ar, 0)];
     const float* bias = params[pidx_cat(ar, 0) + 1];
-    const int ldw = 3 * hl + 252;
+    const int ldw = 3 * hl + ar.ew;
     float* y = ws + w.a[0];
     for (int b = 0; b < 3; ++b)
       if (lin_fwd(st, n, ar.c[0], hl, ws + w.xb[b][ar.nb - 1], hl, W, ldw, b * hl, y, ar.c[0], b > 0, nullptr, 0, 0.f)) return 1;
-    if (lin_fwd(st, n, ar.c[0], 252, E, 252, W, ldw, 3 * hl, y, ar.c[0], 1, bias, 1, 0.01f)) return 1;
+    if (lin_fwd(st, n, ar.c[0], ar.ew, E, ar.ew, W, ldw, 3 * hl, y, ar.c[0], 1, bias, 1, 0.01f)) return 1;
   }
   for (int j = 1; j < ar.nc; ++j) {
     if (lin_fwd(st, n, ar.c[j], ar.c[j - 1], ws + w.a[j - 1], ar.c[j - 1], params[pidx_cat(ar, j)], ar.c[j - 1], 0, ws + w.a[j],
@@ -1115,12 +1129,18 @@ extern "C" int b200nerf_depthnet_train_fwd(const float* const* params, int n_bra
   LAUNCH_CHECK();
   return 0;
 }
+extern "C" int b200nerf_depthnet_train_fwd(const float* const* params, int n_branch, const int* hidden, int n_cat,
+                                           const int* cat_hidden, const float* rays_o, const float* rays_d, int n_rays, float radius,
+                                           float near_, float far_, float* ws, float* out_z, void* stream) {
+  return b200nerf_depthnet_train_fwd_multires(params, n_branch, hidden, n_cat, cat_hidden, 10, rays_o, rays_d, n_rays, radius, near_, far_,
+                                              ws, out_z, stream);
+}
 
 // Weight gradients are split-K sums and bias gradients column sums added atomically: the gradient tensors are zeroed first -- one
 // memset when the caller laid them out back to back (training.py does), else one each.
 static int zero_grads(const DnArch& ar, float* const* grads, cudaStream_t st) {
   std::vector<size_t> numel;
-  const int ed[3] = {63, 63, 126};
+  const int ed[3] = {ar.ed(0), ar.ed(1), ar.ed(2)};
   const int hl = ar.h[ar.nb - 1], cl = ar.c[ar.nc - 1];
   for (int b = 0; b < 3; ++b)
     for (int i = 0; i < ar.nb; ++i) {
@@ -1128,7 +1148,7 @@ static int zero_grads(const DnArch& ar, float* const* grads, cudaStream_t st) {
       numel.push_back(ar.h[i]);
     }
   for (int j = 0; j < ar.nc; ++j) {
-    numel.push_back(static_cast<size_t>(ar.c[j]) * (j == 0 ? 3 * hl + 252 : ar.c[j - 1]));
+    numel.push_back(static_cast<size_t>(ar.c[j]) * (j == 0 ? 3 * hl + ar.ew : ar.c[j - 1]));
     numel.push_back(ar.c[j]);
   }
   numel.push_back(cl);   // the head: its gradients are atomic sums of the fused head kernel
@@ -1150,7 +1170,7 @@ static int zero_grads(const DnArch& ar, float* const* grads, cudaStream_t st) {
 // The collapsed branches' backward behind the ray reduction (G = D^T e, g = D^T 1 already in the workspace): the R recurrence over the
 // weights (writes dV_i, db_i, dU_0), then the 3 (L-1) small dU_i products in one launch.
 static int chain_backward(const DnArch& ar, const DnWs& w, float* ws, const float* const* params, float* const* grads, cudaStream_t st) {
-  const int ed[3] = {63, 63, 126};
+  const int ed[3] = {ar.ed(0), ar.ed(1), ar.ed(2)};
   const ChainParams cp = chain_params(ar, w, ws, params, grads);
   if (chain_configure()) return 1;
   if (launch_chain(chain_bwd_kernel, cp, st)) return 1;
@@ -1177,13 +1197,13 @@ static int chain_backward(const DnArch& ar, const DnWs& w, float* ws, const floa
   return 0;
 }
 
-extern "C" int b200nerf_depthnet_train_bwd(const float* const* params, int n_branch, const int* hidden, int n_cat,
-                                           const int* cat_hidden, int n_rays, float near_, float far_, float* ws, const float* dz,
-                                           float* const* grads, void* stream) {
+extern "C" int b200nerf_depthnet_train_bwd_multires(const float* const* params, int n_branch, const int* hidden, int n_cat,
+                                                    const int* cat_hidden, int multires, int n_rays, float near_, float far_, float* ws,
+                                                    const float* dz, float* const* grads, void* stream) {
   if (n_rays <= 0) return 0;
   if (!params || !ws || !dz || !grads) return b200_fail("b200nerf_depthnet_train_bwd: null argument");
   DnArch ar;
-  if (dn_arch(n_branch, hidden, n_cat, cat_hidden, &ar)) return 1;
+  if (dn_arch(n_branch, hidden, n_cat, cat_hidden, multires, &ar)) return 1;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const int n = n_rays;
   const DnWs w = dn_layout(ar, n);
@@ -1220,9 +1240,9 @@ extern "C" int b200nerf_depthnet_train_bwd(const float* const* params, int n_bra
       g = g2;
       g2 = tmp;
     }
-    const int ed[3] = {63, 63, 126}, eo[3] = {0, 63, 126};
+    const int ed[3] = {ar.ed(0), ar.ed(1), ar.ed(2)}, eo[3] = {ar.eo(0), ar.eo(1), ar.eo(2)};
     const int pc0 = pidx_cat(ar, 0);
-    const int ldw0 = 3 * hl + 252;
+    const int ldw0 = 3 * hl + ar.ew;
     float* cur[3];
     float* alt[3];
     for (int b = 0; b < 3; ++b) {
@@ -1233,7 +1253,7 @@ extern "C" int b200nerf_depthnet_train_bwd(const float* const* params, int n_bra
       GemmProb q[7];
       for (int b = 0; b < 3; ++b)
         q[b] = prob_wgrad(n, ar.c[0], hl, g, ar.c[0], ws + w.xb[b][ar.nb - 1], hl, grads[pc0], ldw0, b * hl, b == 0 ? grads[pc0 + 1] : nullptr, true);
-      q[3] = prob_wgrad(n, ar.c[0], 252, g, ar.c[0], E, 252, grads[pc0], ldw0, 3 * hl, nullptr, true);
+      q[3] = prob_wgrad(n, ar.c[0], ar.ew, g, ar.c[0], E, ar.ew, grads[pc0], ldw0, 3 * hl, nullptr, true);
       for (int b = 0; b < 3; ++b) q[4 + b] = prob_dgrad(n, ar.c[0], hl, g, ar.c[0], params[pc0], ldw0, b * hl, cur[b], hl);
       if (tgemm_group(st, q, 7)) return 1;
     }
@@ -1243,7 +1263,7 @@ extern "C" int b200nerf_depthnet_train_bwd(const float* const* params, int n_bra
       CUDA_TRY(cudaMemsetAsync(ws + w.G[0], 0, (w.gv[2] + CH_MAXH - w.G[0]) * sizeof(float), st));
       GemmProb q[3];
       for (int b = 0; b < 3; ++b)
-        q[b] = prob_wgrad(n, hl, ed[b], cur[b], hl, E + eo[b], 252, ws + w.G[b], CH_LD, 0, ws + w.gv[b], true);
+        q[b] = prob_wgrad(n, hl, ed[b], cur[b], hl, E + eo[b], ar.ew, ws + w.G[b], CH_LD, 0, ws + w.gv[b], true);
       if (tgemm_group(st, q, 3)) return 1;
       if (chain_backward(ar, w, ws, params, grads, st)) return 1;
       return 0;
@@ -1256,10 +1276,10 @@ extern "C" int b200nerf_depthnet_train_bwd(const float* const* params, int n_bra
         const int pb = pidx_branch(ar, b, i);
         const int prev_w = i == 0 ? ed[b] : ar.h[i - 1];
         const float* prev = i == 0 ? e : ws + w.xb[b][i - 1];
-        const int prev_ld = i == 0 ? 252 : ar.h[i - 1];
+        const int prev_ld = i == 0 ? ar.ew : ar.h[i - 1];
         const int ldw = prev_w + ed[b];
         q[nq++] = prob_wgrad(n, ar.h[i], prev_w, cur[b], ar.h[i], prev, prev_ld, grads[pb], ldw, 0, grads[pb + 1], true);
-        q[nq++] = prob_wgrad(n, ar.h[i], ed[b], cur[b], ar.h[i], e, 252, grads[pb], ldw, prev_w, nullptr, true);
+        q[nq++] = prob_wgrad(n, ar.h[i], ed[b], cur[b], ar.h[i], e, ar.ew, grads[pb], ldw, prev_w, nullptr, true);
         if (i > 0) q[nq++] = prob_dgrad(n, ar.h[i], ar.h[i - 1], cur[b], ar.h[i], params[pb], ldw, 0, alt[b], ar.h[i - 1]);
       }
       if (tgemm_group(st, q, nq)) return 1;
@@ -1285,19 +1305,19 @@ extern "C" int b200nerf_depthnet_train_bwd(const float* const* params, int n_bra
       g = g2;
       g2 = tmp;
     } else {
-      const int ldw = 3 * hl + 252;
+      const int ldw = 3 * hl + ar.ew;
       for (int b = 0; b < 3; ++b)
         if (lin_wgrad(st, n, ar.c[0], hl, g, ar.c[0], ws + w.xb[b][ar.nb - 1], hl, grads[pc], ldw, b * hl)) return 1;
-      if (lin_wgrad(st, n, ar.c[0], 252, g, ar.c[0], E, 252, grads[pc], ldw, 3 * hl)) return 1;
+      if (lin_wgrad(st, n, ar.c[0], ar.ew, g, ar.c[0], E, ar.ew, grads[pc], ldw, 3 * hl)) return 1;
     }
   }
   // g = d(pre-activation of cat_layers.0) [n, c0]; branches
   const float* gc0 = g;
   float* gb = g2;                       // gradient of the current branch layer's output ...
   float* gb_alt = ws + w.g2;            // ... and of the layer below it
-  const int ed[3] = {63, 63, 126}, eo[3] = {0, 63, 126};
+  const int ed[3] = {ar.ed(0), ar.ed(1), ar.ed(2)}, eo[3] = {ar.eo(0), ar.eo(1), ar.eo(2)};
   const int pc0 = pidx_cat(ar, 0);
-  const int ldw0 = 3 * hl + 252;
+  const int ldw0 = 3 * hl + ar.ew;
   for (int b = 0; b < 3; ++b) {
     const float* e = E + eo[b];
     // d x_b,last = gc0 * W_cat0[:, b*hl : (b+1)*hl]
@@ -1307,11 +1327,11 @@ extern "C" int b200nerf_depthnet_train_bwd(const float* const* params, int n_bra
       const int pb = pidx_branch(ar, b, i);
       const int prev_w = i == 0 ? ed[b] : ar.h[i - 1];
       const float* prev = i == 0 ? e : ws + w.xb[b][i - 1];
-      const int prev_ld = i == 0 ? 252 : ar.h[i - 1];
+      const int prev_ld = i == 0 ? ar.ew : ar.h[i - 1];
       const int ldw = prev_w + ed[b];
       if (colsum(st, cur, n, ar.h[i], ar.h[i], grads[pb + 1])) return 1;
       if (lin_wgrad(st, n, ar.h[i], prev_w, cur, ar.h[i], prev, prev_ld, grads[pb], ldw, 0)) return 1;
-      if (lin_wgrad(st, n, ar.h[i], ed[b], cur, ar.h[i], e, 252, grads[pb], ldw, prev_w)) return 1;
+      if (lin_wgrad(st, n, ar.h[i], ed[b], cur, ar.h[i], e, ar.ew, grads[pb], ldw, prev_w)) return 1;
       if (i > 0) {
         float* nxt = cur == gb ? gb_alt : gb;
         if (lin_dgrad(st, n, ar.h[i], ar.h[i - 1], cur, ar.h[i], params[pb], ldw, 0, nxt, ar.h[i - 1], 0)) return 1;
@@ -1320,6 +1340,11 @@ extern "C" int b200nerf_depthnet_train_bwd(const float* const* params, int n_bra
     }
   }
   return 0;
+}
+extern "C" int b200nerf_depthnet_train_bwd(const float* const* params, int n_branch, const int* hidden, int n_cat,
+                                           const int* cat_hidden, int n_rays, float near_, float far_, float* ws, const float* dz,
+                                           float* const* grads, void* stream) {
+  return b200nerf_depthnet_train_bwd_multires(params, n_branch, hidden, n_cat, cat_hidden, 10, n_rays, near_, far_, ws, dz, grads, stream);
 }
 
 // ---- the same backward, split at the losses ----------------------------------------------------------------------------------
@@ -1332,12 +1357,13 @@ extern "C" int b200nerf_depthnet_train_bwd(const float* const* params, int n_bra
 static bool split_backward_ok(const DnArch& ar, int n, const float* const* params) {
   return tensor_path_ok(n) && can_collapse(ar, n, params);
 }
-extern "C" int b200nerf_depthnet_train_jac(const float* const* params, int n_branch, const int* hidden, int n_cat, const int* cat_hidden,
-                                           int n_rays, float near_, float far_, float* ws, float* const* grads, void* stream) {
+extern "C" int b200nerf_depthnet_train_jac_multires(const float* const* params, int n_branch, const int* hidden, int n_cat,
+                                                    const int* cat_hidden, int multires, int n_rays, float near_, float far_, float* ws,
+                                                    float* const* grads, void* stream) {
   if (n_rays <= 0) return 0;
   if (!params || !ws || !grads) return b200_fail("b200nerf_depthnet_train_jac: null argument");
   DnArch ar;
-  if (dn_arch(n_branch, hidden, n_cat, cat_hidden, &ar)) return 1;
+  if (dn_arch(n_branch, hidden, n_cat, cat_hidden, multires, &ar)) return 1;
   if (!split_backward_ok(ar, n_rays, params)) return 0;   // b200nerf_depthnet_train_bwd_jac then runs the one-pass backward
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const int n = n_rays;
@@ -1365,10 +1391,14 @@ extern "C" int b200nerf_depthnet_train_jac(const float* const* params, int n_bra
       if (tgemm_group(st, &q, 1)) return 1;
     }
   }
-  const int pc0 = pidx_cat(ar, 0), ldw0 = 3 * hl + 252;
+  const int pc0 = pidx_cat(ar, 0), ldw0 = 3 * hl + ar.ew;
   GemmProb q[3];
   for (int b = 0; b < 3; ++b) q[b] = prob_dgrad(n, ar.c[0], hl, ws + w.jac[0], ar.c[0], params[pc0], ldw0, b * hl, ws + w.gx[2 * b], hl);
   return tgemm_group(st, q, 3);
+}
+extern "C" int b200nerf_depthnet_train_jac(const float* const* params, int n_branch, const int* hidden, int n_cat, const int* cat_hidden,
+                                           int n_rays, float near_, float far_, float* ws, float* const* grads, void* stream) {
+  return b200nerf_depthnet_train_jac_multires(params, n_branch, hidden, n_cat, cat_hidden, 10, n_rays, near_, far_, ws, grads, stream);
 }
 // fork / join events of the split backward's second stream, one pair per device and host thread
 static int fork_events(cudaEvent_t* fork, cudaEvent_t* join) {
@@ -1381,15 +1411,16 @@ static int fork_events(cudaEvent_t* fork, cudaEvent_t* join) {
   *join = ev[dev][1];
   return 0;
 }
-extern "C" int b200nerf_depthnet_train_bwd_jac(const float* const* params, int n_branch, const int* hidden, int n_cat,
-                                               const int* cat_hidden, int n_rays, float near_, float far_, float* ws, const float* dz,
-                                               float* const* grads, void* stream, void* stream_aux) {
+extern "C" int b200nerf_depthnet_train_bwd_jac_multires(const float* const* params, int n_branch, const int* hidden, int n_cat,
+                                                        const int* cat_hidden, int multires, int n_rays, float near_, float far_, float* ws,
+                                                        const float* dz, float* const* grads, void* stream, void* stream_aux) {
   if (n_rays <= 0) return 0;
   if (!params || !ws || !dz || !grads) return b200_fail("b200nerf_depthnet_train_bwd_jac: null argument");
   DnArch ar;
-  if (dn_arch(n_branch, hidden, n_cat, cat_hidden, &ar)) return 1;
+  if (dn_arch(n_branch, hidden, n_cat, cat_hidden, multires, &ar)) return 1;
   if (!split_backward_ok(ar, n_rays, params))
-    return b200nerf_depthnet_train_bwd(params, n_branch, hidden, n_cat, cat_hidden, n_rays, near_, far_, ws, dz, grads, stream);
+    return b200nerf_depthnet_train_bwd_multires(params, n_branch, hidden, n_cat, cat_hidden, multires, n_rays, near_, far_, ws, dz, grads,
+                                                stream);
   cudaStream_t st = static_cast<cudaStream_t>(stream), sa = static_cast<cudaStream_t>(stream_aux);
   const bool fork = sa != nullptr && sa != st;
   const int n = n_rays;
@@ -1397,7 +1428,7 @@ extern "C" int b200nerf_depthnet_train_bwd_jac(const float* const* params, int n
   const float* E = ws + w.E;
   const int cl = ar.c[ar.nc - 1], hl = ar.h[ar.nb - 1];
   const int ph = pidx_head(ar);
-  const int ed[3] = {63, 63, 126}, eo[3] = {0, 63, 126};
+  const int ed[3] = {ar.ed(0), ar.ed(1), ar.ed(2)}, eo[3] = {ar.eo(0), ar.eo(1), ar.eo(2)};
   auto launch_all = [&](std::vector<GemmProb>& q) -> int {
     for (GemmProb& p : q) p.kscale = dz;
     for (size_t i = 0; i < q.size(); i += b200::tg::MAX_PROB) {
@@ -1409,7 +1440,7 @@ extern "C" int b200nerf_depthnet_train_bwd_jac(const float* const* params, int n
   // the branches' one reduction over the rays: G_b = D_b^T e_b, g_b = D_b^T 1 with D_b = dz * (J_0 W_cat0[:, b]) (pre-zeroed by _jac)
   std::vector<GemmProb> qg, q;
   for (int b = 0; b < 3; ++b)
-    qg.push_back(prob_wgrad(n, hl, ed[b], ws + w.gx[2 * b], hl, E + eo[b], 252, ws + w.G[b], CH_LD, 0, ws + w.gv[b], true));
+    qg.push_back(prob_wgrad(n, hl, ed[b], ws + w.gx[2 * b], hl, E + eo[b], ar.ew, ws + w.G[b], CH_LD, 0, ws + w.gv[b], true));
   cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
   if (fork) {
     // The weight-only branch chain (chain_bwd + chain_du: ~100 us on 64 SMs, whatever the batch) needs only G: it runs on the second
@@ -1428,11 +1459,11 @@ extern "C" int b200nerf_depthnet_train_bwd_jac(const float* const* params, int n
     const int pc = pidx_cat(ar, j);
     q.push_back(prob_wgrad(n, ar.c[j], ar.c[j - 1], ws + w.jac[j], ar.c[j], ws + w.a[j - 1], ar.c[j - 1], grads[pc], ar.c[j - 1], 0, grads[pc + 1], true));
   }
-  const int pc0 = pidx_cat(ar, 0), ldw0 = 3 * hl + 252;
+  const int pc0 = pidx_cat(ar, 0), ldw0 = 3 * hl + ar.ew;
   for (int b = 0; b < 3; ++b)
     q.push_back(prob_wgrad(n, ar.c[0], hl, ws + w.jac[0], ar.c[0], ws + w.xb[b][ar.nb - 1], hl, grads[pc0], ldw0, b * hl,
                            b == 0 ? grads[pc0 + 1] : nullptr, true));
-  q.push_back(prob_wgrad(n, ar.c[0], 252, ws + w.jac[0], ar.c[0], E, 252, grads[pc0], ldw0, 3 * hl, nullptr, true));
+  q.push_back(prob_wgrad(n, ar.c[0], ar.ew, ws + w.jac[0], ar.c[0], E, ar.ew, grads[pc0], ldw0, 3 * hl, nullptr, true));
   if (!fork) q.insert(q.end(), qg.begin(), qg.end());
   if (launch_all(q)) return 1;
   if (fork) {
@@ -1440,6 +1471,12 @@ extern "C" int b200nerf_depthnet_train_bwd_jac(const float* const* params, int n
     return 0;
   }
   return chain_backward(ar, w, ws, params, grads, st);
+}
+extern "C" int b200nerf_depthnet_train_bwd_jac(const float* const* params, int n_branch, const int* hidden, int n_cat,
+                                               const int* cat_hidden, int n_rays, float near_, float far_, float* ws, const float* dz,
+                                               float* const* grads, void* stream, void* stream_aux) {
+  return b200nerf_depthnet_train_bwd_jac_multires(params, n_branch, hidden, n_cat, cat_hidden, 10, n_rays, near_, far_, ws, dz, grads, stream,
+                                                  stream_aux);
 }
 
 // ------------------------------------------------------------------------------------------- NeRF at one sample per ray + d/dz
@@ -1865,11 +1902,11 @@ extern "C" int b200nerf_debug_sgemm(int M, int N, int K, const float* A, long sA
 
 /* Which kernels the DepthNet training passes pick for this architecture, batch and parameter alignment, from the same predicates the
    passes call (pure host code: only the pointer VALUES are read, nothing is launched). */
-extern "C" int b200nerf_debug_depthnet_train_route(const float* const* params, int n_branch, const int* hidden, int n_cat,
-                                                   const int* cat_hidden, int n_rays) {
+extern "C" int b200nerf_debug_depthnet_train_route_multires(const float* const* params, int n_branch, const int* hidden, int n_cat,
+                                                            const int* cat_hidden, int multires, int n_rays) {
   if (!params || n_rays < 0) return -b200_fail("b200nerf_debug_depthnet_train_route: bad arguments");
   DnArch ar;
-  if (dn_arch(n_branch, hidden, n_cat, cat_hidden, &ar)) return -1;
+  if (dn_arch(n_branch, hidden, n_cat, cat_hidden, multires, &ar)) return -1;
   for (int v : ar.h)
     if (v < 1) return -b200_fail("b200nerf_debug_depthnet_train_route: branch width %d", v);
   for (int v : ar.c)
@@ -1878,4 +1915,8 @@ extern "C" int b200nerf_debug_depthnet_train_route(const float* const* params, i
   return (can_collapse(ar, n, params) ? B200NERF_ROUTE_COLLAPSED : 0) | (fused_chain_ok(ar, n, params) ? B200NERF_ROUTE_FUSED_CHAIN : 0) |
          (split_cat0(ar, n, params) ? B200NERF_ROUTE_SPLIT_CAT0 : 0) | (split_backward_ok(ar, n, params) ? B200NERF_ROUTE_SPLIT_BACKWARD : 0) |
          (tensor_path_ok(n) ? B200NERF_ROUTE_TENSOR_PATH : 0);
+}
+extern "C" int b200nerf_debug_depthnet_train_route(const float* const* params, int n_branch, const int* hidden, int n_cat,
+                                                   const int* cat_hidden, int n_rays) {
+  return b200nerf_debug_depthnet_train_route_multires(params, n_branch, hidden, n_cat, cat_hidden, 10, n_rays);
 }

@@ -21,8 +21,10 @@ class DepthNet(nn.Module):
                  origin_channels: int = 3, direction_channels: int = 3, multires: int = 10, sphere_radius: float = 2.0,
                  near: int = 2, far: int = 6):
         super().__init__()
-        if origin_channels != 3 or direction_channels != 3 or multires != 10:
-            raise NotImplementedError("the B200 DepthNet kernel implements 3-channel rays with multires=10")
+        if origin_channels != 3 or direction_channels != 3:
+            raise NotImplementedError("the B200 DepthNet kernel implements 3-channel rays")
+        if multires not in packing.MULTIRES_RANGE:
+            raise ValueError(f"multires={multires} out of range: the B200 DepthNet kernels serve multires 1..10")
         self.sphere_radius = torch.tensor([sphere_radius])
         self.near, self.far = near, far
         d3, d6 = 3 * (1 + 2 * multires), 6 * (1 + 2 * multires)
@@ -68,7 +70,8 @@ class DepthNet(nn.Module):
             from .. import training
 
             return training.DepthNetTrainFn.apply(rays_o.contiguous().float(), rays_d.contiguous().float(),
-                                                  training.depthnet_arch(self), float(self.sphere_radius), float(self.near),
+                                                  (*training.depthnet_arch(self), training.depthnet_multires(self)),
+                                                  float(self.sphere_radius), float(self.near),
                                                   float(self.far), *training.depthnet_params(self))
         return ops.depthnet_forward(self.packed(), rays_o, rays_d, float(self.sphere_radius), float(self.near),
                                     float(self.far))

@@ -97,47 +97,65 @@ class PackedNeRF:
             self.aux.data_ptr(), int(self.prec), float(self.guard_kappa))
 
 
+MULTIRES_RANGE = range(1, 11)   # positional-encoding sizes DepthNet's kernels serve: enc(o) is at most 63 <= 64 columns wide
+
+
+def depthnet_multires(origin_in_features: int) -> int:
+    """The ``multires`` m of a DepthNet whose ``origin_layers.0`` takes ``origin_in_features`` = 2 d3 inputs, d3 = 3 (1 + 2m)."""
+    m, rest = divmod(origin_in_features - 6, 12)
+    if rest or m not in MULTIRES_RANGE:
+        raise ValueError(f"origin_layers.0 has {origin_in_features} in_features, which is no DepthNet with multires in 1..10 "
+                         f"(2 * 3 * (1 + 2 * multires))")
+    return m
+
+
 def fold_depthnet(sd: Dict[str, torch.Tensor]):
     """Fold origin/direction/intersection branches and cat_layers[0] into one affine map (fp64).
 
     depth_nets/depth_net.py:136-163: every branch layer is ``x = Linear(cat([x, e]))`` with NO activation, so the
     branch output is affine in its encoding e; cat_layers[0] then sees an affine function of (e_o, e_d, e_i).
     Returns (w0 [256,256], b0 [256], hidden [(W [256,256], b [256])...], head_w [256], head_b [1]) over the
-    kernel's column layout enc(o) | enc(d) | enc(hit_near) | enc(hit_far), 64 columns each (last one zero)."""
+    kernel's column layout enc(o) | enc(d) | enc(hit_near) | enc(hit_far), 64 columns each, of which the first
+    d3 = 3 (1 + 2 multires) are used (multires from ``origin_layers.0.weight``, see depthnet_multires) and the rest zero."""
     d = {k: v.detach().to("cpu", torch.float64) for k, v in sd.items()}
+    m = depthnet_multires(d["origin_layers.0.weight"].shape[1])
+    d3 = 3 * (1 + 2 * m)
 
     def branch(name: str, dim: int):
         w, b = d[f"{name}.0.weight"], d[f"{name}.0.bias"]
         if w.shape[1] != 2 * dim:
-            raise ValueError(f"{name}.0.weight: unexpected in_features {w.shape[1]}")
+            raise ValueError(f"{name}.0.weight: unexpected in_features {w.shape[1]} (multires {m}: {2 * dim})")
         a, c = w[:, :dim] + w[:, dim:], b.clone()
         i = 1
         while f"{name}.{i}.weight" in d:
             w, b = d[f"{name}.{i}.weight"], d[f"{name}.{i}.bias"]
             h = w.shape[1] - dim
+            if h != a.shape[0]:
+                raise ValueError(f"{name}.{i}.weight: unexpected in_features {w.shape[1]} (multires {m}: {a.shape[0] + dim})")
             a, c = w[:, :h] @ a + w[:, h:], w[:, :h] @ c + b
             i += 1
         return a, c
 
-    a_o, c_o = branch("origin_layers", 63)
-    a_d, c_d = branch("direction_layers", 63)
-    a_i, c_i = branch("intersection_layers", 126)
+    a_o, c_o = branch("origin_layers", d3)
+    a_d, c_d = branch("direction_layers", d3)
+    a_i, c_i = branch("intersection_layers", 2 * d3)
     wc, bc = d["cat_layers.0.weight"], d["cat_layers.0.bias"]
     h = a_o.shape[0]
-    if wc.shape[1] != 3 * h + 252 or wc.shape[0] > 256:
-        raise ValueError("cat_layers.0 shape not supported (multires must be 10, width <= 256)")
-    m_o = wc[:, 0:h] @ a_o + wc[:, 3 * h : 3 * h + 63]
-    m_d = wc[:, h : 2 * h] @ a_d + wc[:, 3 * h + 63 : 3 * h + 126]
-    m_i = wc[:, 2 * h : 3 * h] @ a_i + wc[:, 3 * h + 126 : 3 * h + 252]
+    if wc.shape[1] != 3 * h + 4 * d3 or wc.shape[0] > 256:
+        raise ValueError(f"cat_layers.0 shape {tuple(wc.shape)} not supported (multires {m}: in_features {3 * h + 4 * d3}, width <= 256)")
+    e0 = 3 * h
+    m_o = wc[:, 0:h] @ a_o + wc[:, e0 : e0 + d3]
+    m_d = wc[:, h : 2 * h] @ a_d + wc[:, e0 + d3 : e0 + 2 * d3]
+    m_i = wc[:, 2 * h : 3 * h] @ a_i + wc[:, e0 + 2 * d3 : e0 + 4 * d3]
     bias0 = bc + wc[:, 0:h] @ c_o + wc[:, h : 2 * h] @ c_d + wc[:, 2 * h : 3 * h] @ c_i
     n0 = wc.shape[0]
     w0 = torch.zeros(256, 256, dtype=torch.float64)
-    w0[:n0, 0:63] = m_o
-    w0[:n0, 64:127] = m_d
+    w0[:n0, 0:d3] = m_o
+    w0[:n0, 64 : 64 + d3] = m_d
     # 6-wide encoding block q holds [near xyz, far xyz]; regroup per hit point
-    m_i = m_i.reshape(n0, 21, 2, 3)
-    w0[:n0, 128:191] = m_i[:, :, 0, :].reshape(n0, 63)
-    w0[:n0, 192:255] = m_i[:, :, 1, :].reshape(n0, 63)
+    m_i = m_i.reshape(n0, 1 + 2 * m, 2, 3)
+    w0[:n0, 128 : 128 + d3] = m_i[:, :, 0, :].reshape(n0, d3)
+    w0[:n0, 192 : 192 + d3] = m_i[:, :, 1, :].reshape(n0, d3)
     b0 = torch.zeros(256, dtype=torch.float64)
     b0[:n0] = bias0
 
@@ -162,21 +180,23 @@ def fold_depthnet(sd: Dict[str, torch.Tensor]):
 
 
 class PackedDepthNet:
-    """Device image of DepthNet for inference (branches folded, see fold_depthnet)."""
+    """Device image of DepthNet for inference (branches folded, see fold_depthnet); the image records its multires."""
 
     def __init__(self, state_dict: Dict[str, torch.Tensor], device, prec: int = PREC_SPLIT):
         L = _lib.lib()
         w0, b0, hidden, hw, hb = fold_depthnet(state_dict)
+        multires = depthnet_multires(state_dict["origin_layers.0.weight"].shape[1])
         flat = [t for pair in hidden for t in pair]
         n_hidden = len(hidden)
         wpack = torch.empty(L.b200nerf_depthnet_wpack_bytes(n_hidden, prec), dtype=torch.uint8)
         aux = torch.empty(L.b200nerf_depthnet_aux_floats(n_hidden), dtype=torch.float32)
         arr = _ptr_array(flat) if flat else None
         _lib.check(
-            L.b200nerf_depthnet_pack(w0.data_ptr(), b0.data_ptr(), C.cast(arr, C.c_void_p) if flat else None, n_hidden,
-                                     hw.data_ptr(), hb.data_ptr(), prec, wpack.data_ptr(), aux.data_ptr())
+            L.b200nerf_depthnet_pack_multires(w0.data_ptr(), b0.data_ptr(), C.cast(arr, C.c_void_p) if flat else None, n_hidden,
+                                              hw.data_ptr(), hb.data_ptr(), multires, prec, wpack.data_ptr(), aux.data_ptr())
         )
         self.prec = prec
+        self.multires = multires
         self.n_hidden = n_hidden
         self.wpack = wpack.to(device)
         self.aux = aux.to(device)

@@ -35,6 +35,11 @@ def depthnet_arch(module):
     return hidden, cat
 
 
+def depthnet_multires(module) -> int:
+    """The positional-encoding size ``multires`` of a DepthNet shell, from the width of its first origin layer."""
+    return packing.depthnet_multires(module.origin_layers[0].in_features)
+
+
 def depthnet_params(module) -> List[torch.nn.Parameter]:
     """Parameters in the order ``b200nerf_depthnet_train_fwd`` expects (= state_dict order)."""
     out = []
@@ -46,23 +51,25 @@ def depthnet_params(module) -> List[torch.nn.Parameter]:
 
 
 class DepthNetTrainFn(torch.autograd.Function):
-    """z [N,1] = DepthNet(rays_o, rays_d) in literal per-layer fp32 form, differentiable w.r.t. the parameters."""
+    """z [N,1] = DepthNet(rays_o, rays_d) in literal per-layer fp32 form, differentiable w.r.t. the parameters.
+    ``arch`` = (branch widths, cat widths, multires)."""
 
     @staticmethod
     def forward(ctx, rays_o, rays_d, arch, radius, near, far, *params):
-        hidden, cat = arch
+        hidden, cat, multires = arch
         L = _lib.lib()
         n = rays_o.shape[0]
         dev = rays_o.device
         for p in params:
             if p.dtype != torch.float32 or not p.is_cuda or not p.is_contiguous():
                 raise _lib.B200NerfError("DepthNet parameters must be contiguous fp32 CUDA tensors")
-        ws = torch.empty(L.b200nerf_depthnet_train_ws_floats(n, len(hidden), _ints(hidden), len(cat), _ints(cat)), device=dev)
+        ws = torch.empty(L.b200nerf_depthnet_train_ws_floats_multires(n, len(hidden), _ints(hidden), len(cat), _ints(cat), multires),
+                         device=dev)
         z = torch.empty(n, 1, device=dev)
         with torch.cuda.device(dev):
-            _lib.check(L.b200nerf_depthnet_train_fwd(_ptrs(list(params)), len(hidden), _ints(hidden), len(cat), _ints(cat),
-                                                     rays_o.data_ptr(), rays_d.data_ptr(), n, float(radius), float(near),
-                                                     float(far), ws.data_ptr(), z.data_ptr(), _stream()))
+            _lib.check(L.b200nerf_depthnet_train_fwd_multires(_ptrs(list(params)), len(hidden), _ints(hidden), len(cat), _ints(cat),
+                                                              multires, rays_o.data_ptr(), rays_d.data_ptr(), n, float(radius),
+                                                              float(near), float(far), ws.data_ptr(), z.data_ptr(), _stream()))
         ctx.ws, ctx.arch, ctx.nf, ctx.n = ws, arch, (float(near), float(far)), n
         ctx.save_for_backward(*params)
         return z
@@ -70,7 +77,7 @@ class DepthNetTrainFn(torch.autograd.Function):
     @staticmethod
     def backward(ctx, dz):
         params = ctx.saved_tensors
-        hidden, cat = ctx.arch
+        hidden, cat, multires = ctx.arch
         L = _lib.lib()
         dz = dz.contiguous().float()
         # one flat buffer, parameter order: the C side zeroes it with a single memset (its split-K weight gradients and bias
@@ -81,8 +88,9 @@ class DepthNetTrainFn(torch.autograd.Function):
             grads.append(flat[off:off + p.numel()].view_as(p))
             off += p.numel()
         with torch.cuda.device(dz.device):
-            _lib.check(L.b200nerf_depthnet_train_bwd(_ptrs(list(params)), len(hidden), _ints(hidden), len(cat), _ints(cat), ctx.n,
-                                                     ctx.nf[0], ctx.nf[1], ctx.ws.data_ptr(), dz.data_ptr(), _ptrs(grads), _stream()))
+            _lib.check(L.b200nerf_depthnet_train_bwd_multires(_ptrs(list(params)), len(hidden), _ints(hidden), len(cat), _ints(cat),
+                                                              multires, ctx.n, ctx.nf[0], ctx.nf[1], ctx.ws.data_ptr(), dz.data_ptr(),
+                                                              _ptrs(grads), _stream()))
         # the activations in ctx.ws stay valid: the reference back-propagates twice (retain_graph=True, Trainer.py:537-538)
         return (None, None, None, None, None, None) + tuple(grads)
 
@@ -214,6 +222,7 @@ def fused_render_and_backward(trainer, optimizer, render_kwargs, batch_rays, tar
     n, dev = rays_o.shape[0], rays_o.device
     target = target_s.contiguous().float()
     hidden, cat = depthnet_arch(dn)
+    arch = (len(hidden), _ints(hidden), len(cat), _ints(cat), depthnet_multires(dn))
     cache = dn.__dict__.get("_b200_train_cache")
     if cache is None or cache["dev"] != dev or cache["ptrs"] != [p.data_ptr() for p in params]:
         flat = torch.zeros(sum(p.numel() for p in params), device=dev)
@@ -239,7 +248,7 @@ def fused_render_and_backward(trainer, optimizer, render_kwargs, batch_rays, tar
         side = _side_stream(dev) if TARGET_SM_LIMIT > 0 else None
         # every buffer is allocated on the main stream (the side stream only runs kernels between the two wait_stream calls), so the
         # caching allocator never sees a cross-stream hand-off
-        ws = torch.empty(L.b200nerf_depthnet_train_ws_floats(n, len(hidden), _ints(hidden), len(cat), _ints(cat)), device=dev)
+        ws = torch.empty(L.b200nerf_depthnet_train_ws_floats_multires(n, *arch), device=dev)
         z = torch.empty(n, 1, device=dev)
         net_packed = net.packed() if hasattr(net, "packed") else None   # before the fork: a repack allocates and copies on the main stream
         net_params = nerf_params(net)
@@ -248,9 +257,8 @@ def fused_render_and_backward(trainer, optimizer, render_kwargs, batch_rays, tar
         if side is not None:
             side.wait_stream(main)
         st = side.cuda_stream if side is not None else main.cuda_stream
-        _lib.check(L.b200nerf_depthnet_train_fwd(p_arr, len(hidden), _ints(hidden), len(cat), _ints(cat), rays_o.data_ptr(),
-                                                 rays_d.data_ptr(), n, float(dn.sphere_radius), nf[0], nf[1], ws.data_ptr(),
-                                                 z.data_ptr(), st))
+        _lib.check(L.b200nerf_depthnet_train_fwd_multires(p_arr, *arch, rays_o.data_ptr(), rays_d.data_ptr(), n, float(dn.sphere_radius),
+                                                          nf[0], nf[1], ws.data_ptr(), z.data_ptr(), st))
         g_arr = _ptrs(cache["grads"])
         split_bwd = SPLIT_BACKWARD
         side2 = _side_stream(dev, 1) if (side is not None and split_bwd and THIRD_STREAM) else None
@@ -260,8 +268,8 @@ def fused_render_and_backward(trainer, optimizer, render_kwargs, batch_rays, tar
         if split_bwd:
             # the backward's sequential half (input-gradient chain with a unit upstream gradient) needs neither the losses nor the
             # colour path: it runs beside d raw / d z on a third stream
-            _lib.check(L.b200nerf_depthnet_train_jac(p_arr, len(hidden), _ints(hidden), len(cat), _ints(cat), n, nf[0], nf[1],
-                                                     ws.data_ptr(), g_arr, side2.cuda_stream if side2 is not None else st))
+            _lib.check(L.b200nerf_depthnet_train_jac_multires(p_arr, *arch, n, nf[0], nf[1], ws.data_ptr(), g_arr,
+                                                              side2.cuda_stream if side2 is not None else st))
         prev_limit = L.b200nerf_set_sm_limit(TARGET_SM_LIMIT) if side is not None else 0
         try:
             c = trainer.sample_coarse_points(near=hier["near"], far=hier["far"], perturb=kw["perturb"], N_rays=n, N_samples=kw["N_samples"],
@@ -288,11 +296,10 @@ def fused_render_and_backward(trainer, optimizer, render_kwargs, batch_rays, tar
                                          ws2.data_ptr(), losses.data_ptr(), dz.data_ptr(), st))
         if split_bwd:
             aux = side.cuda_stream if (side is not None and FORK_BRANCH_CHAIN) else None   # idle after the join above
-            _lib.check(L.b200nerf_depthnet_train_bwd_jac(p_arr, len(hidden), _ints(hidden), len(cat), _ints(cat), n, nf[0], nf[1],
-                                                         ws.data_ptr(), dz.data_ptr(), g_arr, st, aux))
+            _lib.check(L.b200nerf_depthnet_train_bwd_jac_multires(p_arr, *arch, n, nf[0], nf[1], ws.data_ptr(), dz.data_ptr(), g_arr,
+                                                                  st, aux))
         else:
-            _lib.check(L.b200nerf_depthnet_train_bwd(p_arr, len(hidden), _ints(hidden), len(cat), _ints(cat), n, nf[0], nf[1],
-                                                     ws.data_ptr(), dz.data_ptr(), g_arr, st))
+            _lib.check(L.b200nerf_depthnet_train_bwd_multires(p_arr, *arch, n, nf[0], nf[1], ws.data_ptr(), dz.data_ptr(), g_arr, st))
     for p, g in zip(params, cache["grads"]):
         if p.grad is not g:
             p.grad = g
