@@ -50,15 +50,23 @@ const char* b200nerf_last_error(void);
 
 /* ---- weight packing (host side, run once per checkpoint load / optimizer step) ------------------------- */
 
-/* NeRF(D=8, W=256, input_ch=63, input_ch_views=27, skips=[4], use_viewdirs=True)
- * (nerf_pytorch/run_nerf_helpers.py:67-107).  `h_tensors` = 24 host fp32 pointers in this order:
+/* NeRF(D=8, W=256, input_ch=d, input_ch_views=dv, skips=[4], use_viewdirs=True)
+ * (nerf_pytorch/run_nerf_helpers.py:67-107), d = 3 (1 + 2 multires), dv = 3 (1 + 2 multires_views).
+ * `h_tensors` = 24 host fp32 pointers in this order:
  * pts_linears.0.weight, pts_linears.0.bias, ..., pts_linears.7.{weight,bias}, views_linears.0.{weight,bias},
  * feature_linear.{weight,bias}, alpha_linear.{weight,bias}, rgb_linear.{weight,bias}.
  * Produces the weight-slab stream (`h_wpack`, b200nerf_nerf_wpack_bytes(prec) bytes) and the fp32 bias/head
- * block (`h_aux`, b200nerf_nerf_aux_floats() floats); copy both to the device. */
+ * block (`h_aux`, b200nerf_nerf_aux_floats() floats); copy both to the device.
+ * b200nerf_nerf_pack_multires serves multires 1..10 and multires_views 1..4: gamma(pts) fills the first d of the 64 columns of
+ * its operand block, gamma(viewdir) the first dv of its 32, and the weights of the other columns are zero, so the image has the
+ * size of every other multires.  It records both counts in the aux block, so every NeRF entry point that takes `aux` (render,
+ * query, guard band, b200nerf_nerf_point_jvp_packed) encodes at the image's own sizes.  b200nerf_nerf_pack is the same with
+ * 10 / 4. */
 size_t b200nerf_nerf_wpack_bytes(int prec);
 size_t b200nerf_nerf_aux_floats(void);
 int b200nerf_nerf_pack(const float* const* h_tensors, int prec, void* h_wpack, float* h_aux);
+int b200nerf_nerf_pack_multires(const float* const* h_tensors, int multires, int multires_views, int prec, void* h_wpack,
+                                float* h_aux);
 
 /* DepthNet (depth_nets/depth_net.py:10-169) in inference form.  Its three branches apply no activation
  * (depth_net.py:140,148,156 are no-ops), so branches + cat_layers[0] are one affine map of the encodings.
@@ -115,17 +123,19 @@ int b200nerf_points(const float* rays_o, const float* rays_d, const float* z, in
                     void* stream);
 
 /* Trainer.run_network + NeRF.forward (nerf_pytorch/trainers/Trainer.py:789-806,
- * run_nerf_helpers.py:109-134): positional encoding of the sample positions (63) and view directions (27)
- * fused into the 8x256 skip@4 MLP.  Sample positions are either o + d*z (`z` [n_rays,S], `pts` NULL) or explicit
+ * run_nerf_helpers.py:109-134): positional encoding of the sample positions (d wide, 63 at multires 10) and view directions
+ * (dv wide, 27 at multires_views 4; both sizes from `aux`) fused into the 8x256 skip@4 MLP.  Sample positions are either o + d*z (`z` [n_rays,S], `pts` NULL) or explicit
  * (`pts` [n_rays,S,3]).  out_raw [n_rays,S,4] = (r,g,b,sigma) pre-activation. */
 int b200nerf_nerf_mlp_fwd(const void* wpack, const float* aux, int prec, const float* rays_o, const float* rays_d,
                           const float* viewdirs, const float* z, const float* pts, int n_rays, int S, float* out_raw,
                           void* stream);
 
 /* Single-pass 16-bit image of the same 24 NeRF tensors for the fast kernel (prec = FP16 or BF16):
- * b200nerf_nerf_fast_wpack_bytes() bytes; the fp32 bias/head block is the `h_aux` of b200nerf_nerf_pack. */
+ * b200nerf_nerf_fast_wpack_bytes() bytes; the fp32 bias/head block is the `h_aux` of b200nerf_nerf_pack.  The _multires form
+ * takes the sizes of b200nerf_nerf_pack_multires; its aux block (packed at the same sizes) carries them to the kernel. */
 size_t b200nerf_nerf_fast_wpack_bytes(void);
 int b200nerf_nerf_pack_fast(const float* const* h_tensors, int prec, void* h_wpack);
+int b200nerf_nerf_pack_fast_multires(const float* const* h_tensors, int multires, int multires_views, int prec, void* h_wpack);
 
 /* Same operator as b200nerf_nerf_mlp_fwd on the throughput kernel: two 128-row tiles per SM ping-pong between the
  * tensor core and the epilogue warps, SMs paired as 2-CTA clusters (tcgen05 cta_group::2), one MMA per K16 block.
@@ -279,6 +289,12 @@ int b200nerf_depthnet_train_bwd_jac_multires(const float* const* params, int n_b
 size_t b200nerf_nerf_point_ws_floats(int n_rays);
 int b200nerf_nerf_point_jvp(const float* const* params, const float* rays_o, const float* rays_d, const float* viewdirs,
                             const float* z, int n_rays, float* ws, float* out_raw, float* out_draw_dz, void* stream);
+/* The same at multires 1..10 / multires_views 1..4 (the tensors' shapes: pts_linears.0 [256, d], pts_linears.5 [256, d + 256],
+ * views_linears.0 [128, 256 + dv]); the functions above are these with 10 / 4.  The workspace size returns 0 out of range. */
+size_t b200nerf_nerf_point_ws_floats_multires(int n_rays, int multires, int multires_views);
+int b200nerf_nerf_point_jvp_multires(const float* const* params, int multires, int multires_views, const float* rays_o,
+                                     const float* rays_d, const float* viewdirs, const float* z, int n_rays, float* ws,
+                                     float* out_raw, float* out_draw_dz, void* stream);
 
 /* The same two outputs from the PACKED split-precision model (b200nerf_nerf_pack: bf16 hi + lo operands, three MMAs per block,
  * fp32 accumulate -- the precision of B200NERF_PREC_SPLIT inference) in two launches of the fused tensor-core MLP kernel instead

@@ -26,6 +26,7 @@ SIGNATURES = {
     "b200nerf_nerf_wpack_bytes": (SZ, [I]),
     "b200nerf_nerf_aux_floats": (SZ, []),
     "b200nerf_nerf_pack": (I, [P, I, P, P]),
+    "b200nerf_nerf_pack_multires": (I, [P, I, I, I, P, P]),
     "b200nerf_depthnet_wpack_bytes": (SZ, [I, I]),
     "b200nerf_depthnet_aux_floats": (SZ, [I]),
     "b200nerf_depthnet_pack": (I, [P, P, P, I, P, P, I, P, P]),
@@ -40,6 +41,7 @@ SIGNATURES = {
     "b200nerf_nerf_mlp_fwd": (I, [P, P, I, P, P, P, P, P, I, I, P, P]),
     "b200nerf_nerf_fast_wpack_bytes": (SZ, []),
     "b200nerf_nerf_pack_fast": (I, [P, I, P]),
+    "b200nerf_nerf_pack_fast_multires": (I, [P, I, I, I, P]),
     "b200nerf_nerf_mlp_fast_fwd": (I, [P, P, I, P, P, P, P, P, I, I, P, P, P, I, F, P]),
     "b200nerf_nerf_mlp_guarded_fwd": (I, [P, P, P, I, P, P, P, P, P, I, I, F, P, P, P]),
     "b200nerf_composite_fwd": (I, [P, P, P, P, I, I, I, P, P, P, P, P, P, P]),
@@ -72,6 +74,8 @@ SIGNATURES = {
     "b200nerf_depthnet_train_bwd_jac_multires": (I, [P, I, P, I, P, I, I, F, F, P, P, P, P, P]),
     "b200nerf_nerf_point_ws_floats": (SZ, [I]),
     "b200nerf_nerf_point_jvp": (I, [P, P, P, P, P, I, P, P, P, P]),
+    "b200nerf_nerf_point_ws_floats_multires": (SZ, [I, I, I]),
+    "b200nerf_nerf_point_jvp_multires": (I, [P, I, I, P, P, P, P, I, P, P, P, P]),
     "b200nerf_nerf_point_jvp_packed_ws_bytes": (SZ, [I]),
     "b200nerf_nerf_point_jvp_packed": (I, [P, P, P, P, P, P, I, P, P, P, P]),
     "b200nerf_debug_catchain_img_bytes": (SZ, [I]),

@@ -125,20 +125,22 @@ static exact::XStep xstep(int n1a, int kb1a, int n1b, int kb1b, int n2, int kb2,
   return s;
 }
 
-// views_linears.0 with the activation-free feature_linear folded in: returns W'' [128, 283] = [W_view[:, :256] * W_feature |
+// views_linears.0 with the activation-free feature_linear folded in: returns W'' [128, 256 + dv] = [W_view[:, :256] * W_feature |
 // W_view[:, 256:]] (valid until the next call on this thread) and, if asked, b' = W_view[:, :256] * b_feature + b_view.
-static const float* nerf_fold_view(const float* const* t, float* bias128) {
+// dv = 3 (1 + 2 multires_views) is the width of gamma(viewdir) (27 at multires_views 4).
+static const float* nerf_fold_view(const float* const* t, int dv, float* bias128) {
   static thread_local std::vector<float> wfold;
   const float *Wv = t[16], *bv = t[17], *Wf = t[18], *bf = t[19];
-  wfold.resize(static_cast<size_t>(128) * 283);
+  const int ld = 256 + dv;
+  wfold.resize(static_cast<size_t>(128) * ld);
   for (int r = 0; r < 128; ++r) {
-    const float* wr = Wv + static_cast<size_t>(r) * 283;
+    const float* wr = Wv + static_cast<size_t>(r) * ld;
     for (int k = 0; k < 256; ++k) {
       double a = 0.0;
       for (int j = 0; j < 256; ++j) a += static_cast<double>(wr[j]) * static_cast<double>(Wf[static_cast<size_t>(j) * 256 + k]);
-      wfold[static_cast<size_t>(r) * 283 + k] = static_cast<float>(a);
+      wfold[static_cast<size_t>(r) * ld + k] = static_cast<float>(a);
     }
-    for (int k = 256; k < 283; ++k) wfold[static_cast<size_t>(r) * 283 + k] = wr[k];
+    for (int k = 256; k < ld; ++k) wfold[static_cast<size_t>(r) * ld + k] = wr[k];
     if (bias128) {
       double b = static_cast<double>(bv[r]);
       for (int j = 0; j < 256; ++j) b += static_cast<double>(wr[j]) * static_cast<double>(bf[j]);
@@ -148,8 +150,11 @@ static const float* nerf_fold_view(const float* const* t, float* bias128) {
   return wfold.data();
 }
 
-// NeRF (run_nerf_helpers.py:109-134); t = the 24 tensors in state_dict order (may be null when only the steps are needed)
-static XProgram nerf_xprogram(const float* const* t) {
+// NeRF (run_nerf_helpers.py:109-134); t = the 24 tensors in state_dict order (may be null when only the steps are needed).
+// d = 3 (1 + 2 multires) and dv = 3 (1 + 2 multires_views) are the widths of gamma(pts) and gamma(viewdir): layer 0 is [256, d],
+// the skip layer [256, d + 256] over cat([gamma(pts), h]), views_linears.0 [128, 256 + dv].  The encodings sit in the first d / dv
+// columns of their 64 / 32-column operand blocks, so the steps (and the pack size) are those of every other multires.
+static XProgram nerf_xprogram(const float* const* t, int d = 63, int dv = 27) {
   auto T = [&](int i) { return t ? t[i] : nullptr; };
   XProgram pg;
   auto add = [&](exact::XStep st, int n_out, XSeg a, XSeg b, int n_segs) {
@@ -161,13 +166,13 @@ static XProgram nerf_xprogram(const float* const* t) {
   {
     exact::XStep s0 = xstep(4, exact::ENC_KB, 0, 0, 0, 0, 2, exact::EPI_STORE, exact::ACT_RELU, NERF_B0);
     s0.wait_p = 1;
-    add(s0, 256, XSeg{exact::ENC_KB, 4, T(0), 63, 0, 63}, none, 1);
+    add(s0, 256, XSeg{exact::ENC_KB, 4, T(0), d, 0, d}, none, 1);
   }
   for (int i = 1; i <= 7; ++i) {
     if (i == 5) {
       exact::XStep s5 = xstep(8, 0, 4, exact::ENC_KB, 8, 8, 2, exact::EPI_STORE, exact::ACT_RELU, NERF_B0 + 256 * 5);
       s5.sig_p = 1;   // gamma(pts) is not read after the first range of the skip layer
-      add(s5, 256, XSeg{0, 16, T(10), 319, 63, 256}, XSeg{exact::ENC_KB, 4, T(10), 319, 0, 63}, 2);
+      add(s5, 256, XSeg{0, 16, T(10), 256 + d, d, 256}, XSeg{exact::ENC_KB, 4, T(10), 256 + d, 0, d}, 2);
     } else {
       add(xstep(8, 0, 0, 0, 8, 8, 2, i == 7 ? exact::EPI_STORE_ALPHA : exact::EPI_STORE, exact::ACT_RELU, NERF_B0 + 256 * i), 256,
           XSeg{0, 16, T(2 * i), 256, 0, 256}, none, 1);
@@ -179,8 +184,8 @@ static XProgram nerf_xprogram(const float* const* t) {
     exact::XStep s8 = xstep(8, 0, 2, exact::VIEW_KB, 8, 8, 1, exact::EPI_NERF_OUT, exact::ACT_RELU, NERF_BV);
     s8.wait_v = 1;
     s8.sig_v = 1;
-    const float* wfold = t ? nerf_fold_view(t, nullptr) : nullptr;
-    add(s8, 128, XSeg{0, 16, wfold, 283, 0, 256}, XSeg{exact::VIEW_KB, 2, wfold, 283, 256, 27}, 2);
+    const float* wfold = t ? nerf_fold_view(t, dv, nullptr) : nullptr;
+    add(s8, 128, XSeg{0, 16, wfold, 256 + dv, 0, 256}, XSeg{exact::VIEW_KB, 2, wfold, 256 + dv, 256, dv}, 2);
   }
   return pg;
 }
@@ -369,24 +374,41 @@ extern "C" size_t b200nerf_nerf_wpack_bytes(int prec) {
 }
 extern "C" size_t b200nerf_nerf_aux_floats(void) { return NERF_AUX_FLOATS; }
 
-extern "C" int b200nerf_nerf_pack(const float* const* t, int prec, void* h_wpack, float* h_aux) {
+// gamma(pts) fills at most the 64 columns of its operand block (3 (1 + 2 multires) <= 64), gamma(viewdir) at most its 32
+static int nerf_multires_check(const char* who, int multires, int multires_views) {
+  if (multires < 1 || multires > 10 || multires_views < 1 || multires_views > 4)
+    return fail("%s: multires=%d / multires_views=%d out of range: the NeRF kernels serve multires 1..10 and multires_views 1..4", who,
+                multires, multires_views);
+  return 0;
+}
+
+extern "C" int b200nerf_nerf_pack_multires(const float* const* t, int multires, int multires_views, int prec, void* h_wpack,
+                                           float* h_aux) {
+  if (nerf_multires_check("b200nerf_nerf_pack", multires, multires_views)) return 1;
   if (!t || !h_wpack || !h_aux) return fail("b200nerf_nerf_pack: null argument");
   if (prec != B200NERF_PREC_SPLIT) return fail("b200nerf_nerf_pack: prec must be B200NERF_PREC_SPLIT");
+  const int d = 3 * (1 + 2 * multires), dv = 3 * (1 + 2 * multires_views);
   uint8_t* o = static_cast<uint8_t*>(h_wpack);
   const float* B[8];
   for (int i = 0; i < 8; ++i) B[i] = t[2 * i + 1];
   const float *Bf = t[19], *Wa = t[20], *Ba = t[21], *Wr = t[22], *Br = t[23];
-  const int rc = pack_xprogram(nerf_xprogram(t), o);
+  const int rc = pack_xprogram(nerf_xprogram(t, d, dv), o);
   if (rc) return rc;
   memset(h_aux, 0, NERF_AUX_FLOATS * sizeof(float));
   for (int i = 0; i < 8; ++i) memcpy(h_aux + NERF_B0 + 256 * i, B[i], 256 * sizeof(float));
   memcpy(h_aux + NERF_BF, Bf, 256 * sizeof(float));
-  nerf_fold_view(t, h_aux + NERF_BV);   // the program runs the view layer with feature_linear folded in
+  nerf_fold_view(t, dv, h_aux + NERF_BV);   // the program runs the view layer with feature_linear folded in
   memcpy(h_aux + NERF_WA, Wa, 256 * sizeof(float));
   h_aux[NERF_BA] = Ba[0];
+  // the encoders' octave counts, read by both kernels; 0 means 10 / 4 (images packed before these slots were used)
+  h_aux[NERF_BA + 1] = multires == 10 ? 0.f : static_cast<float>(multires);
+  h_aux[NERF_BA + 2] = multires_views == 4 ? 0.f : static_cast<float>(multires_views);
   memcpy(h_aux + NERF_WR, Wr, 384 * sizeof(float));
   memcpy(h_aux + NERF_BR, Br, 3 * sizeof(float));
   return 0;
+}
+extern "C" int b200nerf_nerf_pack(const float* const* t, int prec, void* h_wpack, float* h_aux) {
+  return b200nerf_nerf_pack_multires(t, 10, 4, prec, h_wpack, h_aux);
 }
 
 
@@ -442,16 +464,19 @@ static uint8_t* pack_step_fast(int N, const FastSeg* segs, int n_segs, bool fp16
 
 extern "C" size_t b200nerf_nerf_fast_wpack_bytes(void) { return fast::WPACK_BYTES; }
 
-extern "C" int b200nerf_nerf_pack_fast(const float* const* t, int prec, void* h_wpack) {
+// The image does not record the octave counts: the kernel reads them from the aux block of b200nerf_nerf_pack_multires, which must
+// be packed from the same tensors at the same multires / multires_views.
+extern "C" int b200nerf_nerf_pack_fast_multires(const float* const* t, int multires, int multires_views, int prec, void* h_wpack) {
+  if (nerf_multires_check("b200nerf_nerf_pack_fast", multires, multires_views)) return 1;
   if (!t || !h_wpack) return fail("b200nerf_nerf_pack_fast: null argument");
   if (prec != B200NERF_PREC_FP16) return fail("b200nerf_nerf_pack_fast: prec must be B200NERF_PREC_FP16");
   const bool fp16 = true;
+  const int d = 3 * (1 + 2 * multires), dv = 3 * (1 + 2 * multires_views);
   uint8_t* o = static_cast<uint8_t*>(h_wpack);
   const float* W[8];
   for (int i = 0; i < 8; ++i) W[i] = t[2 * i];
-  const float *Wv = t[16], *Wf = t[18];
   {
-    const FastSeg sg[1] = {{W[0], 63, 63, 0, 64}};                               // step 0: pts_linears.0 over gamma(pts)
+    const FastSeg sg[1] = {{W[0], d, d, 0, 64}};                                    // step 0: pts_linears.0 over gamma(pts)
     o = pack_step_fast(256, sg, 1, fp16, o);
   }
   for (int i = 1; i <= 4; ++i) {
@@ -459,7 +484,7 @@ extern "C" int b200nerf_nerf_pack_fast(const float* const* t, int prec, void* h_
     o = pack_step_fast(256, sg, 1, fp16, o);
   }
   {
-    const FastSeg sg[2] = {{W[5], 256, 319, 63, 256}, {W[5], 63, 319, 0, 64}};   // step 5: hidden columns, then gamma(pts)
+    const FastSeg sg[2] = {{W[5], 256, 256 + d, d, 256}, {W[5], d, 256 + d, 0, 64}};   // step 5: hidden columns, then gamma(pts)
     o = pack_step_fast(256, sg, 2, fp16, o);
   }
   for (int i = 6; i <= 7; ++i) {
@@ -469,10 +494,10 @@ extern "C" int b200nerf_nerf_pack_fast(const float* const* t, int prec, void* h_
   {
     // step 8: views_linears.0 with feature_linear folded in (no activation between them, run_nerf_helpers.py:116-121):
     //   W' = W_view[:, :256] * W_feature,  b' = W_view[:, :256] * b_feature + b_view   (fp64 sums)
-    // K = [h7 (256) | gamma(viewdir) (27 -> 32) | two all-zero K16 blocks that fill the last ring stage]
+    // K = [h7 (256) | gamma(viewdir) (dv -> 32) | two all-zero K16 blocks that fill the last ring stage]
     float bfold[128];
-    const float* wfold = nerf_fold_view(t, bfold);
-    const FastSeg sg[3] = {{wfold, 256, 283, 0, 256}, {wfold, 27, 283, 256, 32}, {wfold, 0, 283, 0, 32}};
+    const float* wfold = nerf_fold_view(t, dv, bfold);
+    const FastSeg sg[3] = {{wfold, 256, 256 + dv, 0, 256}, {wfold, dv, 256 + dv, 256, 32}, {wfold, 0, 256 + dv, 0, 32}};
     o = pack_step_fast(128, sg, 3, fp16, o);
     memcpy(o, bfold, 128 * sizeof(float));   // fast::FOLD_BIAS_OFF
     o += 128 * sizeof(float);
@@ -480,6 +505,9 @@ extern "C" int b200nerf_nerf_pack_fast(const float* const* t, int prec, void* h_
   if (static_cast<size_t>(o - static_cast<uint8_t*>(h_wpack)) != fast::WPACK_BYTES)
     return fail("b200nerf_nerf_pack_fast: internal size mismatch");
   return 0;
+}
+extern "C" int b200nerf_nerf_pack_fast(const float* const* t, int prec, void* h_wpack) {
+  return b200nerf_nerf_pack_fast_multires(t, 10, 4, prec, h_wpack);
 }
 
 // the exact kernel keeps all biases + the head in its 3080-float shared-memory block: up to 10 hidden layers (the reference's

@@ -256,6 +256,45 @@ __device__ __noinline__ void depthnet_encode_img_lt10(int nf, const float (&o)[3
   }
 }
 
+// NeRF at multires 1..9 / multires_views 1..3, out of line like depthnet_encode_img_lt10 (octaves j < NF as at NF = 10 / 4)
+__device__ __noinline__ void nerf_encode_pts_lt10(int nf, float x0, float x1, float x2, uint8_t* dst) {
+  const float x[3] = {x0, x1, x2};   // by value: the call keeps the caller's registers off the stack
+  switch (nf) {
+    case 1: encode_store<1, 8>(x, dst); break;
+    case 2: encode_store<2, 8>(x, dst); break;
+    case 3: encode_store<3, 8>(x, dst); break;
+    case 4: encode_store<4, 8>(x, dst); break;
+    case 5: encode_store<5, 8>(x, dst); break;
+    case 6: encode_store<6, 8>(x, dst); break;
+    case 7: encode_store<7, 8>(x, dst); break;
+    case 8: encode_store<8, 8>(x, dst); break;
+    default: encode_store<9, 8>(x, dst); break;
+  }
+}
+__device__ __noinline__ void nerf_encode_tangent_lt10(int nf, float x0, float x1, float x2, float d0, float d1, float d2,
+                                                      uint8_t* dst) {
+  const float x[3] = {x0, x1, x2}, d[3] = {d0, d1, d2};
+  switch (nf) {
+    case 1: encode_tangent_store<1, 8>(x, d, dst); break;
+    case 2: encode_tangent_store<2, 8>(x, d, dst); break;
+    case 3: encode_tangent_store<3, 8>(x, d, dst); break;
+    case 4: encode_tangent_store<4, 8>(x, d, dst); break;
+    case 5: encode_tangent_store<5, 8>(x, d, dst); break;
+    case 6: encode_tangent_store<6, 8>(x, d, dst); break;
+    case 7: encode_tangent_store<7, 8>(x, d, dst); break;
+    case 8: encode_tangent_store<8, 8>(x, d, dst); break;
+    default: encode_tangent_store<9, 8>(x, d, dst); break;
+  }
+}
+__device__ __noinline__ void nerf_encode_view_lt4(int nv, float v0, float v1, float v2, uint8_t* dst) {
+  const float v[3] = {v0, v1, v2};
+  switch (nv) {
+    case 1: encode_store<1, 4>(v, dst); break;
+    case 2: encode_store<2, 4>(v, dst); break;
+    default: encode_store<3, 4>(v, dst); break;
+  }
+}
+
 // eight consecutive floats as ONE 256-bit store (STG.E.256: a full 32-byte sector per lane and instruction; the rows of a tile are
 // 1 KB apart, so the lanes of a warp can never share a sector)
 __device__ __forceinline__ void st_global_v8(float* p, const float (&x)[8]) {
@@ -595,8 +634,17 @@ __global__ void __launch_bounds__(THREADS, 1) mlp_exact_kernel(const __grid_cons
           mbar_wait_lean(free_p_addr, (u - 1) & 1u);    // the previous tile's skip layer no longer reads gamma(pts)
           tc_fence_after();
         }
-        if (INPUT == IN_NERF_TAN) encode_tangent_store<10, 8>(x, dir, act + ENC_KB * 2 * KC_STRIDE + row_off);
-        else encode_store<10, 8>(x, act + ENC_KB * 2 * KC_STRIDE + row_off);
+        // the image's octave counts sit in the aux slots after the alpha-head bias (0 = 10 / 4, images packed before the slots were
+        // used); uniform over the kernel: 10 / 4 run the inline encoders, the smaller sizes the out-of-line ones
+        const int nf = static_cast<int>(saux[p.head_b_off + 1]), nv = static_cast<int>(saux[p.head_b_off + 2]);
+        uint8_t* enc_dst = act + ENC_KB * 2 * KC_STRIDE + row_off;
+        if (nf == 0 || nf == 10) {
+          if (INPUT == IN_NERF_TAN) encode_tangent_store<10, 8>(x, dir, enc_dst);
+          else encode_store<10, 8>(x, enc_dst);
+        } else {
+          if (INPUT == IN_NERF_TAN) nerf_encode_tangent_lt10(nf, x[0], x[1], x[2], dir[0], dir[1], dir[2], enc_dst);
+          else nerf_encode_pts_lt10(nf, x[0], x[1], x[2], enc_dst);
+        }
         fence_proxy_async_smem();
         __syncwarp();
         if (lane == 0) mbar_arrive_remote(rp_bar);
@@ -608,8 +656,10 @@ __global__ void __launch_bounds__(THREADS, 1) mlp_exact_kernel(const __grid_cons
           const float zero8[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
 #pragma unroll
           for (int ch = 0; ch < 4; ++ch) store_split8(act + VIEW_KB * 2 * KC_STRIDE + row_off + ch * KC_STRIDE, zero8);
-        } else {
+        } else if (nv == 0 || nv == 4) {
           encode_store<4, 4>(v, act + VIEW_KB * 2 * KC_STRIDE + row_off);
+        } else {
+          nerf_encode_view_lt4(nv, v[0], v[1], v[2], act + VIEW_KB * 2 * KC_STRIDE + row_off);
         }
         fence_proxy_async_smem();
         __syncwarp();

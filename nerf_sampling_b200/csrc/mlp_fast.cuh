@@ -1,7 +1,8 @@
 // Fused NeRF MLP, single-pass 16-bit operands (fp16 or bf16, fp32 accumulate) on tcgen05 tensor cores (sm_100a).
 //
 // Reference semantics: Trainer.run_network (nerf_pytorch/trainers/Trainer.py:789-806) + NeRF.forward
-// (nerf_pytorch/run_nerf_helpers.py:109-134): gamma(pts) 63-wide, gamma(viewdirs) 27-wide, 8x256 ReLU trunk
+// (nerf_pytorch/run_nerf_helpers.py:109-134): gamma(pts) 3 (1 + 2 multires) wide (63 at multires 10, up to 64), gamma(viewdirs)
+// 3 (1 + 2 multires_views) wide (27 at 4, up to 32), 8x256 ReLU trunk
 // with the input re-concatenated at layer 5, alpha head, feature layer, 128-wide view layer, rgb head.
 //
 // Throughput design (one persistent CTA per SM, SMs paired as 2-CTA clusters):
@@ -176,6 +177,33 @@ __device__ __forceinline__ void encode_store(const float (&x)[3], uint8_t* dst /
       else v[i] = 0.f;
     }
     store8<FP16>(dst + ch * KC_STRIDE, v);
+  }
+}
+
+// multires 1..9 / multires_views 1..3, out of line: their encoders stay out of the kernel's hot code.  For j < NF the octave
+// values are computed exactly as at NF = 10 / 4 (octave 5 accurate when NF > 5).
+template <bool FP16>
+__device__ __noinline__ void encode_pts_lt10(int nf, float x0, float x1, float x2, uint8_t* dst) {
+  const float x[3] = {x0, x1, x2};   // by value: the call keeps the caller's registers off the stack
+  switch (nf) {
+    case 1: encode_store<FP16, 1, 8>(x, dst); break;
+    case 2: encode_store<FP16, 2, 8>(x, dst); break;
+    case 3: encode_store<FP16, 3, 8>(x, dst); break;
+    case 4: encode_store<FP16, 4, 8>(x, dst); break;
+    case 5: encode_store<FP16, 5, 8>(x, dst); break;
+    case 6: encode_store<FP16, 6, 8>(x, dst); break;
+    case 7: encode_store<FP16, 7, 8>(x, dst); break;
+    case 8: encode_store<FP16, 8, 8>(x, dst); break;
+    default: encode_store<FP16, 9, 8>(x, dst); break;
+  }
+}
+template <bool FP16>
+__device__ __noinline__ void encode_view_lt4(int nv, float v0, float v1, float v2, uint8_t* dst) {
+  const float v[3] = {v0, v1, v2};
+  switch (nv) {
+    case 1: encode_store<FP16, 1, 4>(v, dst); break;
+    case 2: encode_store<FP16, 2, 4>(v, dst); break;
+    default: encode_store<FP16, 3, 4>(v, dst); break;
   }
 }
 
@@ -530,6 +558,10 @@ nerf_fast_kernel(const __grid_constant__ FastParams p, const __grid_constant__ T
     const uint32_t view_free_addr = tail_addr + offsetof(Tail, view_free);
     const uint32_t enc_bar = mapa_u32(tail_addr + offsetof(Tail, enc_ready), 0);
     const uint32_t view_bar = mapa_u32(tail_addr + offsetof(Tail, view_ready), 0);
+    // the image's octave counts sit in the aux slots after the alpha-head bias (0 = 10 / 4, images packed before the slots were
+    // used); uniform over the kernel: 10 / 4 run the inline encoders, the smaller sizes the out-of-line ones
+    const int nf = static_cast<int>(sf32[SF_BA + 1]), nv = static_cast<int>(sf32[SF_BA + 2]);
+    const bool nf_full = nf == 0 || nf == 10, nv_full = nv == 0 || nv == 4;
     uint32_t cp[2] = {0, 0}, cw[2] = {0, 0};
     bool first = true;
     for (int u = cluster_id; u < n_units; u += n_clusters) {
@@ -553,7 +585,9 @@ nerf_fast_kernel(const __grid_constant__ FastParams p, const __grid_constant__ T
           mbar_wait_sleepy(pts_free_addr + slot * 8u, cp[slot]++ & 1u, 500);   // the previous tile's skip layer has retired
           tc_fence_after();
         }
-        encode_store<FP16, 10, 8>(x, act + slot * TILE_ACT_BYTES + ENC_KB * 2 * KC_STRIDE + row_off);
+        uint8_t* enc_dst = act + slot * TILE_ACT_BYTES + ENC_KB * 2 * KC_STRIDE + row_off;
+        if (nf_full) encode_store<FP16, 10, 8>(x, enc_dst);
+        else encode_pts_lt10<FP16>(nf, x[0], x[1], x[2], enc_dst);
         fence_proxy_async_smem();
         __syncwarp();
         if (lane == 0) mbar_arrive_remote(enc_bar + slot * 8u);
@@ -569,7 +603,9 @@ nerf_fast_kernel(const __grid_constant__ FastParams p, const __grid_constant__ T
           mbar_wait_sleepy(view_free_addr + slot * 8u, cw[slot]++ & 1u, 500);  // the previous tile's view layer has retired
           tc_fence_after();
         }
-        encode_store<FP16, 4, 4>(v, act + slot * TILE_ACT_BYTES + VIEW_KB * 2 * KC_STRIDE + row_off);
+        uint8_t* view_dst = act + slot * TILE_ACT_BYTES + VIEW_KB * 2 * KC_STRIDE + row_off;
+        if (nv_full) encode_store<FP16, 4, 4>(v, view_dst);
+        else encode_view_lt4<FP16>(nv, v[0], v[1], v[2], view_dst);
         fence_proxy_async_smem();
         __syncwarp();
         if (lane == 0) mbar_arrive_remote(view_bar + slot * 8u);

@@ -1480,21 +1480,23 @@ extern "C" int b200nerf_depthnet_train_bwd_jac(const float* const* params, int n
 }
 
 // ------------------------------------------------------------------------------------------- NeRF at one sample per ray + d/dz
-// rows 0..n-1 = primal gamma(p), rows n..2n-1 = tangent d gamma(p) / dz, p = o + d z; view encoding [n, 27].  Six threads per ray:
-// three position channels (10 sincosf each) and three view-direction channels (4 each).
+// rows 0..n-1 = primal gamma(p), rows n..2n-1 = tangent d gamma(p) / dz, p = o + d z, row width d = 3 (1 + 2 nf); view encoding
+// [n, dv], dv = 3 (1 + 2 nv).  Six threads per ray: three position channels (nf sincosf each) and three view-direction channels (nv).
 __global__ void nerf_point_encode_kernel(const float* __restrict__ ro, const float* __restrict__ rd, const float* __restrict__ vd,
-                                         const float* __restrict__ z, int n, float* __restrict__ enc, float* __restrict__ venc) {
+                                         const float* __restrict__ z, int n, int nf, int nv, float* __restrict__ enc,
+                                         float* __restrict__ venc) {
   const int t = blockIdx.x * blockDim.x + threadIdx.x;
   const int i = t / 6, c = t % 3;
   if (i >= n) return;
   if (t % 6 < 3) {
+    const int d3 = 3 * (1 + 2 * nf);
     const float d = rd[i * 3 + c];
     const float x = __fadd_rn(ro[i * 3 + c], __fmul_rn(d, z[i]));
-    float* p = enc + static_cast<size_t>(i) * 63;
-    float* tg = enc + static_cast<size_t>(n + i) * 63;
+    float* p = enc + static_cast<size_t>(i) * d3;
+    float* tg = enc + static_cast<size_t>(n + i) * d3;
     p[c] = x;
     tg[c] = d;
-    for (int j = 0; j < 10; ++j) {
+    for (int j = 0; j < nf; ++j) {
       const float f = static_cast<float>(1 << j);
       float s, co;
       sincosf(x * f, &s, &co);
@@ -1505,9 +1507,9 @@ __global__ void nerf_point_encode_kernel(const float* __restrict__ ro, const flo
     }
   } else {
     const float v = vd[i * 3 + c];
-    float* e = venc + static_cast<size_t>(i) * 27;
+    float* e = venc + static_cast<size_t>(i) * (3 * (1 + 2 * nv));
     e[c] = v;
-    for (int j = 0; j < 4; ++j) {
+    for (int j = 0; j < nv; ++j) {
       float s, co;
       sincosf(v * static_cast<float>(1 << j), &s, &co);
       e[3 + j * 6 + c] = s;
@@ -1578,26 +1580,42 @@ __global__ void nerf_point_heads_kernel(const float* __restrict__ h7, const floa
   }
 }
 
-extern "C" size_t b200nerf_nerf_point_ws_floats(int n_rays) {
+static bool nerf_point_multires_ok(int multires, int multires_views) {
+  return multires >= 1 && multires <= 10 && multires_views >= 1 && multires_views <= 4;
+}
+// the layout holds the widest encodings (d <= 64, dv <= 32), so the size does not depend on multires / multires_views
+extern "C" size_t b200nerf_nerf_point_ws_floats_multires(int n_rays, int multires, int multires_views) {
+  if (!nerf_point_multires_ok(multires, multires_views)) {
+    b200_fail("b200nerf_nerf_point_ws_floats: multires=%d / multires_views=%d out of range (multires 1..10, multires_views 1..4)",
+              multires, multires_views);
+    return 0;
+  }
   const size_t n = static_cast<size_t>(n_rays);
   return 2 * n * 64 + n * 32 + 3 * (2 * n * 256) + 2 * n * 4 + 2 * n + 256;
 }
+extern "C" size_t b200nerf_nerf_point_ws_floats(int n_rays) { return b200nerf_nerf_point_ws_floats_multires(n_rays, 10, 4); }
 
-// params: the 24 fp32 device tensors of NeRF in state_dict order (see b200nerf_nerf_pack)
-extern "C" int b200nerf_nerf_point_jvp(const float* const* t, const float* rays_o, const float* rays_d, const float* viewdirs,
-                                       const float* z, int n_rays, float* ws, float* out_raw, float* out_draw_dz, void* stream) {
+// params: the 24 fp32 device tensors of NeRF in state_dict order (see b200nerf_nerf_pack) at multires / multires_views:
+// pts_linears.0 is [256, d], pts_linears.5 [256, d + 256], views_linears.0 [128, 256 + dv]
+extern "C" int b200nerf_nerf_point_jvp_multires(const float* const* t, int multires, int multires_views, const float* rays_o,
+                                                const float* rays_d, const float* viewdirs, const float* z, int n_rays, float* ws,
+                                                float* out_raw, float* out_draw_dz, void* stream) {
+  if (!nerf_point_multires_ok(multires, multires_views))
+    return b200_fail("b200nerf_nerf_point_jvp: multires=%d / multires_views=%d out of range (multires 1..10, multires_views 1..4)",
+                     multires, multires_views);
   if (n_rays <= 0) return 0;
   if (!t || !rays_o || !rays_d || !viewdirs || !z || !ws || !out_raw || !out_draw_dz) return b200_fail("b200nerf_nerf_point_jvp: null argument");
+  const int d = 3 * (1 + 2 * multires), dv = 3 * (1 + 2 * multires_views), ld5 = 256 + d, ldv = 256 + dv;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const int n = n_rays, n2 = 2 * n_rays;
-  float* enc = ws;                                   // [2n, 63]
-  float* venc = enc + static_cast<size_t>(n2) * 64;  // [n, 27]
+  float* enc = ws;                                   // [2n, d]
+  float* venc = enc + static_cast<size_t>(n2) * 64;  // [n, dv]
   float* h0 = venc + static_cast<size_t>(n) * 32;    // [2n, 256]
   float* h1 = h0 + static_cast<size_t>(n2) * 256;
   float* h2 = h1 + static_cast<size_t>(n2) * 256;
   float* rgb2 = h2 + static_cast<size_t>(n2) * 256;  // [2n, 3]
   float* al2 = rgb2 + static_cast<size_t>(n2) * 4;   // [2n]
-  nerf_point_encode_kernel<<<(6 * n + 191) / 192, 192, 0, st>>>(rays_o, rays_d, viewdirs, z, n, enc, venc);
+  nerf_point_encode_kernel<<<(6 * n + 191) / 192, 192, 0, st>>>(rays_o, rays_d, viewdirs, z, n, multires, multires_views, enc, venc);
   LAUNCH_CHECK();
   auto act = [&](float* Y, const float* bias, int M, int relu) -> int {
     const size_t tot = static_cast<size_t>(n) * M;
@@ -1615,14 +1633,14 @@ extern "C" int b200nerf_nerf_point_jvp(const float* const* t, const float* rays_
     float* ht[2] = {h1, h1 + blk};          // tangent ping-pong
     float* feat = h2;                       // feature_linear(h7) primal, then its tangent next to it
     float* feat_t = h2 + blk;
-    const float* enc_t = enc + static_cast<size_t>(n) * 63;
+    const float* enc_t = enc + static_cast<size_t>(n) * d;
     auto primal = [&](int layer, const float* x, float* y) {
       GemmProb q = prob_fwd(n, 256, y, 256, t[2 * layer + 1], 1, 0.f);
       if (layer == 0) {
-        seg_fwd(q, enc, 63, t[0], 63, 0, 63);
+        seg_fwd(q, enc, d, t[0], d, 0, d);
       } else if (layer == 5) {
-        seg_fwd(q, enc, 63, t[10], 319, 0, 63);
-        seg_fwd(q, x, 256, t[10], 319, 63, 256);
+        seg_fwd(q, enc, d, t[10], ld5, 0, d);
+        seg_fwd(q, x, 256, t[10], ld5, d, 256);
       } else {
         seg_fwd(q, x, 256, t[2 * layer], 256, 0, 256);
       }
@@ -1634,10 +1652,10 @@ extern "C" int b200nerf_nerf_point_jvp(const float* const* t, const float* rays_
       q.ld_dact = 256;
       q.slope = 0.f;
       if (layer == 0) {
-        seg_fwd(q, enc_t, 63, t[0], 63, 0, 63);
+        seg_fwd(q, enc_t, d, t[0], d, 0, d);
       } else if (layer == 5) {
-        seg_fwd(q, enc_t, 63, t[10], 319, 0, 63);
-        seg_fwd(q, xt, 256, t[10], 319, 63, 256);
+        seg_fwd(q, enc_t, d, t[10], ld5, 0, d);
+        seg_fwd(q, xt, 256, t[10], ld5, d, 256);
       } else {
         seg_fwd(q, xt, 256, t[2 * layer], 256, 0, 256);
       }
@@ -1665,8 +1683,8 @@ extern "C" int b200nerf_nerf_point_jvp(const float* const* t, const float* rays_
       // views_linears.0 on cat([feature, gamma(viewdir)]) + ReLU; feature tangent = W_f t7 (no mask)
       GemmProb q[2];
       q[0] = prob_fwd(n, 128, hv, 128, t[17], 1, 0.f);
-      seg_fwd(q[0], feat, 256, t[16], 283, 0, 256);
-      seg_fwd(q[0], venc, 27, t[16], 283, 256, 27);
+      seg_fwd(q[0], feat, 256, t[16], ldv, 0, 256);
+      seg_fwd(q[0], venc, dv, t[16], ldv, 256, dv);
       q[1] = prob_fwd(n, 256, feat_t, 256, nullptr, 0, 0.f);
       seg_fwd(q[1], ht[1], 256, t[18], 256, 0, 256);
       if (tgemm_group(st, q, 2)) return 1;
@@ -1676,7 +1694,7 @@ extern "C" int b200nerf_nerf_point_jvp(const float* const* t, const float* rays_
       q.dact = hv;
       q.ld_dact = 128;
       q.slope = 0.f;
-      seg_fwd(q, feat_t, 256, t[16], 283, 0, 256);
+      seg_fwd(q, feat_t, 256, t[16], ldv, 0, 256);
       if (tgemm_group(st, &q, 1)) return 1;
     }
     // alpha_linear(h7) / rgb_linear(hv) and their tangents: eight dot products per ray, one warp per ray
@@ -1687,12 +1705,12 @@ extern "C" int b200nerf_nerf_point_jvp(const float* const* t, const float* rays_
   float* cur = h0;
   float* nxt = h1;
   // run_nerf_helpers.py:109-134: h = relu(L_i(h)); after layer 4, h = cat([input_pts, h])
-  if (lin_fwd(st, n2, 256, 63, enc, 63, t[0], 63, 0, cur, 256, 0, nullptr, 0, 0.f)) return 1;
+  if (lin_fwd(st, n2, 256, d, enc, d, t[0], d, 0, cur, 256, 0, nullptr, 0, 0.f)) return 1;
   if (act(cur, t[1], 256, 1)) return 1;
   for (int i = 1; i < 8; ++i) {
     if (i == 5) {
-      if (lin_fwd(st, n2, 256, 63, enc, 63, t[10], 319, 0, nxt, 256, 0, nullptr, 0, 0.f)) return 1;
-      if (lin_fwd(st, n2, 256, 256, cur, 256, t[10], 319, 63, nxt, 256, 1, nullptr, 0, 0.f)) return 1;
+      if (lin_fwd(st, n2, 256, d, enc, d, t[10], ld5, 0, nxt, 256, 0, nullptr, 0, 0.f)) return 1;
+      if (lin_fwd(st, n2, 256, 256, cur, 256, t[10], ld5, d, nxt, 256, 1, nullptr, 0, 0.f)) return 1;
     } else {
       if (lin_fwd(st, n2, 256, 256, cur, 256, t[2 * i], 256, 0, nxt, 256, 0, nullptr, 0, 0.f)) return 1;
     }
@@ -1706,13 +1724,18 @@ extern "C" int b200nerf_nerf_point_jvp(const float* const* t, const float* rays_
   if (lin_fwd(st, n2, 256, 256, cur, 256, t[18], 256, 0, nxt, 256, 0, nullptr, 0, 0.f)) return 1;
   if (act(nxt, t[19], 256, 0)) return 1;
   // views_linears.0 on cat([feature, gamma(viewdir)]): the view part has no tangent
-  if (lin_fwd(st, n2, 128, 256, nxt, 256, t[16], 283, 0, h2, 128, 0, nullptr, 0, 0.f)) return 1;
-  if (lin_fwd(st, n, 128, 27, venc, 27, t[16], 283, 256, h2, 128, 1, nullptr, 0, 0.f)) return 1;
+  if (lin_fwd(st, n2, 128, 256, nxt, 256, t[16], ldv, 0, h2, 128, 0, nullptr, 0, 0.f)) return 1;
+  if (lin_fwd(st, n, 128, dv, venc, dv, t[16], ldv, 256, h2, 128, 1, nullptr, 0, 0.f)) return 1;
   if (act(h2, t[17], 128, 1)) return 1;
   if (lin_fwd(st, n2, 3, 128, h2, 128, t[22], 128, 0, rgb2, 3, 0, nullptr, 0, 0.f)) return 1;
   nerf_point_out_kernel<<<(n + 255) / 256, 256, 0, st>>>(rgb2, al2, t[23], t[21], n, out_raw, out_draw_dz);
   LAUNCH_CHECK();
   return 0;
+}
+
+extern "C" int b200nerf_nerf_point_jvp(const float* const* t, const float* rays_o, const float* rays_d, const float* viewdirs,
+                                       const float* z, int n_rays, float* ws, float* out_raw, float* out_draw_dz, void* stream) {
+  return b200nerf_nerf_point_jvp_multires(t, 10, 4, rays_o, rays_d, viewdirs, z, n_rays, ws, out_raw, out_draw_dz, stream);
 }
 
 // ------------------------------------------------------------------------------------------- Adam

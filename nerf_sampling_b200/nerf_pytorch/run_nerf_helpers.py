@@ -51,6 +51,10 @@ def get_embedder(multires, i=0, input_dims=4):
     return e, e.out_dim
 
 
+_INPUT_CH = {3 * (1 + 2 * m) for m in packing.NERF_MULTIRES_RANGE}
+_INPUT_CH_VIEWS = {3 * (1 + 2 * m) for m in packing.NERF_MULTIRES_VIEWS_RANGE}
+
+
 class NeRF(nn.Module):
     """Parameter shell of the 8x256 skip@4 view-dependent NeRF MLP (run_nerf_helpers.py:67-134)."""
 
@@ -74,12 +78,19 @@ class NeRF(nn.Module):
         self._packed = None
         self._packed_key = None
 
+    def multires(self):
+        """(multires, multires_views) of this net's encodings: input_ch = 3 (1 + 2 multires), input_ch_views likewise."""
+        self._check_supported()
+        return (self.input_ch - 3) // 6, (self.input_ch_views - 3) // 6
+
     def _check_supported(self):
-        if not (self.D == 8 and self.W == 256 and self.input_ch == 63 and self.input_ch_views == 27
+        if not (self.D == 8 and self.W == 256 and self.input_ch in _INPUT_CH and self.input_ch_views in _INPUT_CH_VIEWS
                 and list(self.skips) == [4] and self.use_viewdirs):
             raise NotImplementedError(
-                "the B200 kernel implements NeRF(D=8, W=256, input_ch=63, input_ch_views=27, skips=[4], "
-                "use_viewdirs=True) -- the only configuration experiments/run.py and render.py build")
+                "the B200 kernel implements NeRF(D=8, W=256, input_ch=3*(1+2*multires), input_ch_views=3*(1+2*multires_views), "
+                "skips=[4], use_viewdirs=True) with multires in 1..10 and multires_views in 1..4 (the positional encodings of "
+                f"experiments/run.py and render.py); got D={self.D}, W={self.W}, input_ch={self.input_ch}, "
+                f"input_ch_views={self.input_ch_views}, skips={list(self.skips)}, use_viewdirs={self.use_viewdirs}")
 
     def packed(self) -> PackedNeRF:
         """Packed weight image for the current parameter values (rebuilt when a parameter changes)."""

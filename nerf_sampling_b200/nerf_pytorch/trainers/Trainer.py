@@ -244,8 +244,15 @@ class Trainer:
 
         The encodings described by ``embed_fn`` / ``embeddirs_fn`` are fused into the MLP kernel and the whole batch
         is one launch, so ``netchunk`` has nothing left to bound."""
-        if getattr(embed_fn, "multires", 10) != 10 or getattr(embeddirs_fn, "multires", 4) != 4 or viewdirs is None:
-            raise NotImplementedError("the fused kernel implements multires=10 / multires_views=4 with view directions")
+        if viewdirs is None:
+            raise NotImplementedError("the fused kernel implements the NeRF with view directions (use_viewdirs=True)")
+        # the network's shapes fix the encodings; an embedder that states its size must agree with them
+        m, mv = fn.multires()
+        for name, e, want in (("embed_fn", embed_fn, m), ("embeddirs_fn", embeddirs_fn, mv)):
+            got = getattr(e, "multires", None)
+            if got is not None and got != want:
+                raise ValueError(f"{name} encodes {got} octaves but the network was built for {want} "
+                                 f"(multires {m}, multires_views {mv})")
         lead = list(inputs.shape[:-1])
         pts = inputs.reshape(viewdirs.shape[0], -1, 3)
         raw = fn.query(viewdirs, pts=pts)

@@ -2,7 +2,7 @@
 
 ``PackedNeRF`` / ``PackedDepthNet`` take reference-layout ``state_dict``s (the ``200000.tar`` keys,
 nerf_pytorch/utils.py:59-122) and hold the device-side slab stream + fp32 bias/head block.  Packing itself is
-done by the C ABI (``b200nerf_nerf_pack`` / ``b200nerf_depthnet_pack``); the only arithmetic here is the fp64
+done by the C ABI (``b200nerf_nerf_pack_multires`` / ``b200nerf_depthnet_pack_multires``); the only arithmetic here is the fp64
 folding of DepthNet's activation-free branches into its first dense layer.
 """
 
@@ -24,10 +24,36 @@ NERF_KEYS = (
     [f"pts_linears.{i}.{w}" for i in range(8) for w in ("weight", "bias")]
     + [f"{n}.{w}" for n in ("views_linears.0", "feature_linear", "alpha_linear", "rgb_linear") for w in ("weight", "bias")]
 )
-NERF_SHAPES = {
-    "pts_linears.0.weight": (256, 63), "pts_linears.5.weight": (256, 319), "views_linears.0.weight": (128, 283),
-    "feature_linear.weight": (256, 256), "alpha_linear.weight": (1, 256), "rgb_linear.weight": (3, 128),
-}
+NERF_MULTIRES_RANGE = range(1, 11)        # gamma(pts) is 3 (1 + 2 multires) <= 64 columns: its operand block
+NERF_MULTIRES_VIEWS_RANGE = range(1, 5)   # gamma(viewdir) is 3 (1 + 2 multires_views) <= 32 columns
+
+
+def nerf_shapes(multires: int = 10, multires_views: int = 4) -> Dict[str, tuple]:
+    """The weight shapes of NeRF(D=8, W=256, input_ch=3(1+2 multires), input_ch_views=3(1+2 multires_views), skips=[4])."""
+    d, dv = 3 * (1 + 2 * multires), 3 * (1 + 2 * multires_views)
+    return {"pts_linears.0.weight": (256, d), "pts_linears.5.weight": (256, 256 + d), "views_linears.0.weight": (128, 256 + dv),
+            "feature_linear.weight": (256, 256), "alpha_linear.weight": (1, 256), "rgb_linear.weight": (3, 128)}
+
+
+def _octaves(width: int, what: str, name: str, rng: range) -> int:
+    m, rest = divmod(width - 3, 6)
+    if rest or m not in rng:
+        raise ValueError(f"{what} is {width} wide, which is no encoding the NeRF kernels serve: 3 * (1 + 2 * {name}) with {name} "
+                         f"in {rng.start}..{rng.stop - 1}")
+    return m
+
+
+def nerf_multires(state_dict: Dict[str, torch.Tensor]):
+    """(multires, multires_views) of a NeRF state_dict, from pts_linears.0 (input_ch = 3 (1 + 2 multires)) and views_linears.0
+    (256 + input_ch_views); pts_linears.5 must agree (256 + input_ch), as must every other shape."""
+    m = _octaves(state_dict["pts_linears.0.weight"].shape[-1], "gamma(pts) (pts_linears.0 in_features)", "multires",
+                 NERF_MULTIRES_RANGE)
+    mv = _octaves(state_dict["views_linears.0.weight"].shape[-1] - 256, "gamma(viewdir) (views_linears.0 in_features - 256)",
+                  "multires_views", NERF_MULTIRES_VIEWS_RANGE)
+    for k, shp in nerf_shapes(m, mv).items():
+        if tuple(state_dict[k].shape) != shp:
+            raise ValueError(f"{k} has shape {tuple(state_dict[k].shape)}, expected {shp} (multires {m}, multires_views {mv})")
+    return m, mv
 
 
 _GENERATION = 0
@@ -62,16 +88,16 @@ def _ptr_array(tensors: List[torch.Tensor]):
 
 
 class PackedNeRF:
-    """Device image of NeRF(D=8, W=256, input_ch=63, input_ch_views=27, skips=[4], use_viewdirs=True)."""
+    """Device image of NeRF(D=8, W=256, input_ch=3(1+2m), input_ch_views=3(1+2mv), skips=[4], use_viewdirs=True), m = multires in
+    1..10 and mv = multires_views in 1..4 (from the weight shapes, see nerf_multires); the aux block records both for the kernels."""
 
     def __init__(self, state_dict: Dict[str, torch.Tensor], device, prec: int = PREC_SPLIT):
         L = _lib.lib()
         for k in NERF_KEYS:
             if k not in state_dict:
                 raise KeyError(f"NeRF state_dict lacks {k!r}: only the 8x256 skip@4 view-dependent model is supported")
-        for k, shp in NERF_SHAPES.items():
-            if tuple(state_dict[k].shape) != shp:
-                raise ValueError(f"{k} has shape {tuple(state_dict[k].shape)}, expected {shp}")
+        self.multires, self.multires_views = nerf_multires(state_dict)
+        mr = (self.multires, self.multires_views)
         host = [_host_f32(state_dict[k]) for k in NERF_KEYS]
         arr = C.cast(_ptr_array(host), C.c_void_p)
         aux = torch.empty(L.b200nerf_nerf_aux_floats(), dtype=torch.float32)
@@ -79,12 +105,12 @@ class PackedNeRF:
         self.wpack = None       # split-precision stream of the exact kernel (mlp_exact.cuh): PREC_SPLIT and the guard band of PREC_FAST
         self.wpack_fast = None  # single-pass fp16 stream of the throughput kernel (mlp_fast.cuh)
         wpack = torch.empty(L.b200nerf_nerf_wpack_bytes(PREC_SPLIT), dtype=torch.uint8)
-        _lib.check(L.b200nerf_nerf_pack(arr, PREC_SPLIT, wpack.data_ptr(), aux.data_ptr()))   # also fills the fp32 bias / head block
+        _lib.check(L.b200nerf_nerf_pack_multires(arr, *mr, PREC_SPLIT, wpack.data_ptr(), aux.data_ptr()))   # also the fp32 bias / head block
         if prec != PREC_FP16:
             self.wpack = wpack.to(device)
         if prec in (PREC_FP16, PREC_FAST):
             wf = torch.empty(L.b200nerf_nerf_fast_wpack_bytes(), dtype=torch.uint8)
-            _lib.check(L.b200nerf_nerf_pack_fast(arr, PREC_FP16, wf.data_ptr()))
+            _lib.check(L.b200nerf_nerf_pack_fast_multires(arr, *mr, PREC_FP16, wf.data_ptr()))
             self.wpack_fast = wf.to(device)
         self.aux = aux.to(device)
         self.guard_kappa = GUARD_KAPPA

@@ -112,9 +112,11 @@ def nerf_point_jvp(packed, params, rays_o, rays_d, viewdirs, z_flat, raw, draw, 
                                                     viewdirs.data_ptr(), z_flat.data_ptr(), n, ws.data_ptr(), raw.data_ptr(),
                                                     draw.data_ptr(), stream))
         return ws
-    ws = torch.empty(L.b200nerf_nerf_point_ws_floats(n), device=dev)
-    _lib.check(L.b200nerf_nerf_point_jvp(_ptrs(list(params)), rays_o.data_ptr(), rays_d.data_ptr(), viewdirs.data_ptr(),
-                                         z_flat.data_ptr(), n, ws.data_ptr(), raw.data_ptr(), draw.data_ptr(), stream))
+    # the packed route reads the encodings' sizes from its aux block; this one takes them from the tensors' shapes
+    mr = packing.nerf_multires(dict(zip(packing.NERF_KEYS, params)))
+    ws = torch.empty(L.b200nerf_nerf_point_ws_floats_multires(n, *mr), device=dev)
+    _lib.check(L.b200nerf_nerf_point_jvp_multires(_ptrs(list(params)), *mr, rays_o.data_ptr(), rays_d.data_ptr(), viewdirs.data_ptr(),
+                                                  z_flat.data_ptr(), n, ws.data_ptr(), raw.data_ptr(), draw.data_ptr(), stream))
     return ws
 
 
