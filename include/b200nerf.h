@@ -122,6 +122,17 @@ int b200nerf_place_samples(const float* mean, const float* offsets, int n_rays, 
 int b200nerf_points(const float* rays_o, const float* rays_d, const float* z, int n_rays, int S, float* out_pts,
                     void* stream);
 
+/* Backward of sample_points_around_mean (nerf_pytorch/utils.py:220-244) w.r.t. `mean`: every placed depth is mean + a constant,
+ * so out_g_mean [n_rays] = sum_s g_z[ray, s], except that uniform mode drops the samples torch.clip(z, clip_lo, clip_hi) cut:
+ * the mask is clip_lo <= mean + offset <= clip_hi (inclusive, on the UNclipped value; a sample clipped onto a bound gets no
+ * gradient).  Gaussian mode has no mask (offsets may be NULL); depth_only (S == 1) is the identity.  Arguments as in
+ * b200nerf_place_samples; g_z [n_rays, S]. */
+int b200nerf_place_samples_bwd(const float* mean, const float* offsets, int n_rays, int S, int mode, float clip_lo, float clip_hi,
+                               const float* g_z, float* out_g_mean, void* stream);
+
+/* Backward of b200nerf_points w.r.t. z: out_g_z [n_rays,S] = sum_k g_pts[ray,s,k] rays_d[ray,k]. */
+int b200nerf_points_bwd(const float* rays_d, const float* g_pts, int n_rays, int S, float* out_g_z, void* stream);
+
 /* Trainer.run_network + NeRF.forward (nerf_pytorch/trainers/Trainer.py:789-806,
  * run_nerf_helpers.py:109-134): positional encoding of the sample positions (d wide, 63 at multires 10) and view directions
  * (dv wide, 27 at multires_views 4; both sizes from `aux`) fused into the 8x256 skip@4 MLP.  Sample positions are either o + d*z (`z` [n_rays,S], `pts` NULL) or explicit
@@ -171,6 +182,18 @@ int b200nerf_nerf_query(const b200nerf_nerf_model* nerf, const float* rays_o, co
 int b200nerf_composite_fwd(const float* raw, const float* z, const float* rays_d, const float* noise, int n_rays,
                            int S, int white_bkgd, float* out_rgb, float* out_disp, float* out_acc, float* out_depth,
                            float* out_weights, float* out_alphas, void* stream);
+
+/* Reverse-mode derivative of DepthNetTrainer.raw2outputs (trainers/sampling_trainer.py:153-230) for S >= 2 (S == 1 has no
+ * intervals; its colour is sigmoid(raw rgb)).  Inputs as in b200nerf_composite_fwd; upstream gradients g_rgb [n_rays,3],
+ * g_disp / g_acc / g_depth [n_rays], g_weights / g_alphas [n_rays,S] -- each may be NULL, meaning zero.  Writes out_g_raw
+ * [n_rays,S,4] (sigmoid' on the colour channels; relu'(sigma + noise) times d alpha / d relu on sigma, relu'(0) = 0) and out_g_z
+ * [n_rays,S] (through dists = (z_{i+1} - z_i) |rays_d| and depth = sum w z; the 1e10 last interval does not depend on z).  The
+ * transmittance term is a reverse scan in double, R_i = g_{i+1} alpha_{i+1} + t_{i+1} R_{i+1}, g_alpha_i = T_i (g_w_i - R_i), with
+ * no division by t = 1 - alpha + 1e-10, so the gradient survives where T underflows in fp32.  disp = 1 / max(1e-10, q) sends
+ * the gradient to q = depth / (acc + 1e-10) where q > 1e-10 (half of it on a tie), like torch.max. */
+int b200nerf_composite_bwd(const float* raw, const float* z, const float* rays_d, const float* noise, int n_rays, int S,
+                           int white_bkgd, const float* g_rgb, const float* g_disp, const float* g_acc, const float* g_depth,
+                           const float* g_weights, const float* g_alphas, float* out_g_raw, float* out_g_z, void* stream);
 
 /* Same arithmetic, image-tile output: out_rgbd [n_rays,4] = (r, g, b, disp) per ray -- the layout the multi-GPU render
  * all-gathers (one 16-byte pixel per ray, SURVEY.md 8(e)), written by the kernel itself instead of two copy launches. */
@@ -295,6 +318,13 @@ size_t b200nerf_nerf_point_ws_floats_multires(int n_rays, int multires, int mult
 int b200nerf_nerf_point_jvp_multires(const float* const* params, int multires, int multires_views, const float* rays_o,
                                      const float* rays_d, const float* viewdirs, const float* z, int n_rays, float* ws,
                                      float* out_raw, float* out_draw_dz, void* stream);
+/* The same at S samples per ray (Trainer.run_network on o + d z, run_nerf_helpers.py:109-134, differentiated along z):
+ * z [n_rays,S], out_raw / out_draw_dz [n_rays*S,4]; the sample points are the rows and row r uses ray r / S.  The functions above
+ * are these with S = 1.  ws: b200nerf_nerf_samples_ws_floats_multires(n_rays, S, ...) floats (0 on bad arguments). */
+size_t b200nerf_nerf_samples_ws_floats_multires(int n_rays, int S, int multires, int multires_views);
+int b200nerf_nerf_samples_jvp_multires(const float* const* params, int multires, int multires_views, const float* rays_o,
+                                       const float* rays_d, const float* viewdirs, const float* z, int n_rays, int S, float* ws,
+                                       float* out_raw, float* out_draw_dz, void* stream);
 
 /* The same two outputs from the PACKED split-precision model (b200nerf_nerf_pack: bf16 hi + lo operands, three MMAs per block,
  * fp32 accumulate -- the precision of B200NERF_PREC_SPLIT inference) in two launches of the fused tensor-core MLP kernel instead
@@ -304,6 +334,17 @@ size_t b200nerf_nerf_point_jvp_packed_ws_bytes(int n_rays);
 int b200nerf_nerf_point_jvp_packed(const void* wpack, const float* aux, const float* rays_o, const float* rays_d,
                                    const float* viewdirs, const float* z, int n_rays, void* ws, float* out_raw,
                                    float* out_draw_dz, void* stream);
+/* The same at S samples per ray: z [n_rays,S], out_raw / out_draw_dz [n_rays*S,4]; the masks are MAX_STEPS x n_rays*S x 4
+ * words (b200nerf_nerf_samples_jvp_packed_ws_bytes(n_rays, S) bytes).  The two functions above are these with S = 1. */
+size_t b200nerf_nerf_samples_jvp_packed_ws_bytes(int n_rays, int S);
+int b200nerf_nerf_samples_jvp_packed(const void* wpack, const float* aux, const float* rays_o, const float* rays_d,
+                                     const float* viewdirs, const float* z, int n_rays, int S, void* ws, float* out_raw,
+                                     float* out_draw_dz, void* stream);
+/* raw and its Jacobian w.r.t. EXPLICIT sample points (Trainer.run_network(pts, ...), Trainer.py:789-806): pts [n_rays,S,3],
+ * viewdirs [n_rays,3]; one primal pass with masks, then three tangent passes along the unit axes.  out_raw [n_rays*S,4],
+ * out_draw_dpts [n_rays*S,3,4] (d raw / d x, y, z); ws as for b200nerf_nerf_samples_jvp_packed. */
+int b200nerf_nerf_pts_jvp_packed(const void* wpack, const float* aux, const float* pts, const float* viewdirs, int n_rays, int S,
+                                 void* ws, float* out_raw, float* out_draw_dpts, void* stream);
 
 /* torch.optim.Adam (no weight decay, no amsgrad) on one tensor; the gradient is multiplied by grad_scale first
  * (1/world_size after a sum all-reduce).  step counts from 1. */

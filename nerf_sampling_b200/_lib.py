@@ -46,6 +46,9 @@ SIGNATURES = {
     "b200nerf_nerf_mlp_guarded_fwd": (I, [P, P, P, I, P, P, P, P, P, I, I, F, P, P, P]),
     "b200nerf_composite_fwd": (I, [P, P, P, P, I, I, I, P, P, P, P, P, P, P]),
     "b200nerf_composite_tile_fwd": (I, [P, P, P, P, I, I, I, P, P, P, P, P, P]),
+    "b200nerf_composite_bwd": (I, [P, P, P, P, I, I, I, P, P, P, P, P, P, P, P, P]),
+    "b200nerf_place_samples_bwd": (I, [P, P, I, I, I, F, F, P, P, P]),
+    "b200nerf_points_bwd": (I, [P, P, I, I, P, P]),
     "b200nerf_render_depthnet_tile": (I, [P, P, I, I, P, P, P, P, I, I, I, P, F, F, F, P, P, P, P, P, P, P, P, P]),
     "b200nerf_set_sm_limit": (I, [I]),
     "b200nerf_nerf_query": (I, [P, P, P, P, P, P, I, I, P, P, P]),
@@ -78,6 +81,11 @@ SIGNATURES = {
     "b200nerf_nerf_point_jvp_multires": (I, [P, I, I, P, P, P, P, I, P, P, P, P]),
     "b200nerf_nerf_point_jvp_packed_ws_bytes": (SZ, [I]),
     "b200nerf_nerf_point_jvp_packed": (I, [P, P, P, P, P, P, I, P, P, P, P]),
+    "b200nerf_nerf_samples_ws_floats_multires": (SZ, [I, I, I, I]),
+    "b200nerf_nerf_samples_jvp_multires": (I, [P, I, I, P, P, P, P, I, I, P, P, P, P]),
+    "b200nerf_nerf_samples_jvp_packed_ws_bytes": (SZ, [I, I]),
+    "b200nerf_nerf_samples_jvp_packed": (I, [P, P, P, P, P, P, I, I, P, P, P, P]),
+    "b200nerf_nerf_pts_jvp_packed": (I, [P, P, P, P, I, I, P, P, P, P]),
     "b200nerf_debug_catchain_img_bytes": (SZ, [I]),
     "b200nerf_debug_catchain_pack": (I, [P, P, P, P, I, P, P, P, P]),
     "b200nerf_train_loss": (I, [P, P, P, P, P, I, P, P, P, P]),

@@ -1037,6 +1037,176 @@ extern "C" int b200nerf_composite_tile_fwd(const float* raw, const float* z, con
                         out_alphas, 4, 4, stream);
 }
 
+// ------------------------------------------------------------------------------------------- compositing backward
+// The reverse-mode derivative of raw2outputs (trainers/sampling_trainer.py:153-230) for S >= 2, one warp per ray, sample
+// i0 + lane in pass i0.  The forward's per-sample arithmetic is recomputed bit for bit (alpha, t = 1 - alpha + 1e-10, the 1e10 last
+// interval).  With gw_i the total gradient reaching w_i and R_i = sum_{j>i} gw_j alpha_j prod_{i<l<j} t_l,
+//   g_alpha_i = g_alphas_i + T_i (gw_i - R_i),   R_i = gw_{i+1} alpha_{i+1} + t_{i+1} R_{i+1},   R_{S-1} = 0,
+// a reverse scan (in double, like the forward's cumprod) that never divides by t, so it keeps the gradient where T underflows.
+// Pass 1 (ascending) forms T_i as the forward does and parks it in out_g_z; pass 2 (descending) reads it back, runs the scan and
+// overwrites out_g_z with d/dz.  dist_j = (z_{j+1} - z_j) |rays_d| feeds z_{j+1} and z_j; lane 0's z-gradient waits for the
+// term of the pass below it (`pend`).
+__device__ __forceinline__ float comp_alpha(float sg, float dist, float* e) {
+  *e = expf(__fmul_rn(-fmaxf(sg, 0.f), dist));
+  return __fadd_rn(1.0f, -*e);
+}
+
+__global__ void __launch_bounds__(256) composite_bwd_kernel(
+    const float* __restrict__ raw, const float* __restrict__ z, const float* __restrict__ rays_d, const float* __restrict__ noise,
+    int n_rays, int S, int white, const float* __restrict__ g_rgb, const float* __restrict__ g_disp, const float* __restrict__ g_acc,
+    const float* __restrict__ g_depth, const float* __restrict__ g_weights, const float* __restrict__ g_alphas,
+    float* __restrict__ out_g_raw, float* __restrict__ out_g_z) {
+  const int ray = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  const int lane = threadIdx.x & 31;
+  if (ray >= n_rays) return;   // whole warp leaves together
+  const size_t base = static_cast<size_t>(ray) * S;
+  const float dx = __ldg(rays_d + ray * 3), dy = __ldg(rays_d + ray * 3 + 1), dz = __ldg(rays_d + ray * 3 + 2);
+  const float nrm = __fsqrt_rn(__fadd_rn(__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)), __fmul_rn(dz, dz)));
+  auto sample = [&](int i, float4& rw, float& zi, float& alpha, float& e, float& dist, float& sg) {
+    rw = __ldg(reinterpret_cast<const float4*>(raw) + base + i);
+    zi = __ldg(z + base + i);
+    dist = __fmul_rn(i + 1 < S ? __fadd_rn(__ldg(z + base + i + 1), -zi) : 1e10f, nrm);
+    sg = noise ? __fadd_rn(rw.w, __ldg(noise + base + i)) : rw.w;
+    alpha = comp_alpha(sg, dist, &e);
+  };
+
+  // pass 1: T_i (exclusive cumprod of t, double), acc and depth for the disparity's derivative
+  double carry = 1.0, acc = 0.0, depth = 0.0;
+  for (int i0 = 0; i0 < S; i0 += 32) {
+    const int i = i0 + lane;
+    float4 rw;
+    float zi = 0.f, alpha = 0.f, e, dist, sg;
+    double incl = 1.0;
+    if (i < S) {
+      sample(i, rw, zi, alpha, e, dist, sg);
+      incl = static_cast<double>(__fadd_rn(__fadd_rn(1.0f, -alpha), 1e-10f));
+    }
+#pragma unroll
+    for (int off = 1; off < 32; off <<= 1) {
+      const double v = __shfl_up_sync(0xffffffffu, incl, off);
+      if (lane >= off) incl *= v;
+    }
+    double excl = __shfl_up_sync(0xffffffffu, incl, 1);
+    if (lane == 0) excl = 1.0;
+    const float T = static_cast<float>(carry * excl);
+    carry *= __shfl_sync(0xffffffffu, incl, 31);
+    if (i < S) {
+      const float w = __fmul_rn(alpha, T);
+      out_g_z[base + i] = T;
+      acc += w;
+      depth += static_cast<double>(w) * zi;
+    }
+  }
+#pragma unroll
+  for (int off = 16; off > 0; off >>= 1) {
+    acc += __shfl_xor_sync(0xffffffffu, acc, off);
+    depth += __shfl_xor_sync(0xffffffffu, depth, off);
+  }
+
+  // upstream gradients folded into one coefficient per output: rgb_k = sum w c_k + white (1 - acc), disp = 1 / max(1e-10, q),
+  // q = depth / (acc + 1e-10) (torch.max sends the gradient to the larger argument, half of it on a tie)
+  float gr[3] = {0.f, 0.f, 0.f};
+  if (g_rgb)
+#pragma unroll
+    for (int k = 0; k < 3; ++k) gr[k] = __ldg(g_rgb + ray * 3 + k);
+  double gacc = g_acc ? static_cast<double>(__ldg(g_acc + ray)) : 0.0;
+  double gdep = g_depth ? static_cast<double>(__ldg(g_depth + ray)) : 0.0;
+  if (white) gacc -= static_cast<double>(gr[0]) + gr[1] + gr[2];
+  if (g_disp) {
+    const double den = acc + 1e-10;
+    const double q = depth / den;
+    const double m = static_cast<double>(fmaxf(1e-10f, static_cast<float>(q)));
+    const double share = q > 1e-10 ? 1.0 : (q == 1e-10 ? 0.5 : 0.0);
+    const double gq = -static_cast<double>(__ldg(g_disp + ray)) / (m * m) * share;
+    gdep += gq / den;
+    gacc -= gq * depth / (den * den);
+  }
+
+  // pass 2: reverse scan of R, from the last pass down
+  double R_in = 0.0;   // R of the last sample of the pass being processed (R_{S-1} = 0)
+  float pend = 0.f;    // z-gradient of the previous pass's first sample, short of the dist term of the sample in front of it
+  const int last0 = ((S - 1) >> 5) << 5;
+  for (int i0 = last0; i0 >= 0; i0 -= 32) {
+    const int i = i0 + lane;
+    const bool in = i < S;
+    float4 rw = make_float4(0.f, 0.f, 0.f, 0.f);
+    float zi = 0.f, alpha = 0.f, e = 1.f, dist = 0.f, sg = 0.f, T = 0.f;
+    double t = 1.0, a = 0.0;   // f_i(R) = a_i + t_i R maps R_i onto R_{i-1}
+    float gw = 0.f, c[3] = {0.f, 0.f, 0.f};
+    if (in) {
+      sample(i, rw, zi, alpha, e, dist, sg);
+      T = out_g_z[base + i];
+      t = static_cast<double>(__fadd_rn(__fadd_rn(1.0f, -alpha), 1e-10f));
+      c[0] = 1.0f / (1.0f + expf(-rw.x));
+      c[1] = 1.0f / (1.0f + expf(-rw.y));
+      c[2] = 1.0f / (1.0f + expf(-rw.z));
+      double g = gacc + gdep * zi + static_cast<double>(gr[0]) * c[0] + static_cast<double>(gr[1]) * c[1] +
+                 static_cast<double>(gr[2]) * c[2];
+      if (g_weights) g += __ldg(g_weights + base + i);
+      gw = static_cast<float>(g);
+      a = static_cast<double>(gw) * alpha;
+    }
+    // suffix composition F_l = f_l o f_{l+1} o ... o f_31 as (M, B): F(R) = B + M R
+    double M = t, B = a;
+#pragma unroll
+    for (int off = 1; off < 32; off <<= 1) {
+      const double Mo = __shfl_down_sync(0xffffffffu, M, off), Bo = __shfl_down_sync(0xffffffffu, B, off);
+      if (lane + off < 32) {
+        B = B + M * Bo;
+        M = M * Mo;
+      }
+    }
+    double Mx = __shfl_down_sync(0xffffffffu, M, 1), Bx = __shfl_down_sync(0xffffffffu, B, 1);
+    if (lane == 31) {
+      Mx = 1.0;
+      Bx = 0.0;
+    }
+    const double Ri = Bx + Mx * R_in;                               // R_i
+    const double R_next = __shfl_sync(0xffffffffu, B + M * R_in, 0);   // R_{i0-1}
+
+    float gdist = 0.f, gzi = 0.f;
+    if (in) {
+      float ga = static_cast<float>(static_cast<double>(T) * (static_cast<double>(gw) - Ri));
+      if (g_alphas) ga += __ldg(g_alphas + base + i);
+      // alpha = 1 - e, e = exp(-relu(sg) dist): d alpha / d relu = e dist, d alpha / d dist = e relu; relu'(0) = 0
+      const float ge = __fmul_rn(ga, e);
+      const float gs = sg > 0.f ? __fmul_rn(ge, dist) : 0.f;
+      gdist = i + 1 < S ? __fmul_rn(ge, fmaxf(sg, 0.f)) : 0.f;
+      const float w = __fmul_rn(alpha, T);
+      float4 o;
+      o.x = gr[0] * w * c[0] * (1.0f - c[0]);
+      o.y = gr[1] * w * c[1] * (1.0f - c[1]);
+      o.z = gr[2] * w * c[2] * (1.0f - c[2]);
+      o.w = gs;
+      reinterpret_cast<float4*>(out_g_raw)[base + i] = o;
+      gzi = static_cast<float>(gdep * w) - gdist * nrm;
+    }
+    // + dist_{i-1}'s term: from the lane below, or (lane 0) from the next pass down
+    const float from_below = __shfl_up_sync(0xffffffffu, gdist, 1);
+    if (lane > 0 && in) gzi += from_below * nrm;
+    const float top = __shfl_sync(0xffffffffu, gdist, 31);   // dist_{i0+31} feeds z_{i0+32}: the previous pass's first sample
+    if (lane == 0 && i0 != last0) out_g_z[base + i0 + 32] = pend + top * nrm;
+    pend = __shfl_sync(0xffffffffu, gzi, 0);
+    if (lane > 0 && in) out_g_z[base + i] = gzi;
+    R_in = R_next;
+  }
+  if (lane == 0) out_g_z[base] = pend;
+}
+
+extern "C" int b200nerf_composite_bwd(const float* raw, const float* z, const float* rays_d, const float* noise, int n_rays, int S,
+                                      int white_bkgd, const float* g_rgb, const float* g_disp, const float* g_acc, const float* g_depth,
+                                      const float* g_weights, const float* g_alphas, float* out_g_raw, float* out_g_z, void* stream) {
+  if (n_rays < 0) return fail("b200nerf_composite_bwd: bad sizes n_rays=%d", n_rays);
+  if (S < 2) return fail("b200nerf_composite_bwd: S=%d; S >= 2 is required (S == 1 has no intervals: its colour is sigmoid(raw rgb))", S);
+  if (n_rays == 0) return 0;
+  if (!raw || !z || !rays_d || !out_g_raw || !out_g_z) return fail("b200nerf_composite_bwd: null argument");
+  const int wpb = 8;
+  composite_bwd_kernel<<<(n_rays + wpb - 1) / wpb, wpb * 32, 0, static_cast<cudaStream_t>(stream)>>>(
+      raw, z, rays_d, noise, n_rays, S, white_bkgd, g_rgb, g_disp, g_acc, g_depth, g_weights, g_alphas, out_g_raw, out_g_z);
+  LAUNCH_CHECK();
+  return 0;
+}
+
 // ------------------------------------------------------------------------------------------- MLP launches
 // row_index / n_rows_dev != nullptr: evaluate only the listed sample points (at most list_cap of them), in place
 static int nerf_exact_launch(const void* wpack, const float* aux, const float* rays_o, const float* rays_d, const float* viewdirs,
@@ -1062,37 +1232,81 @@ static int nerf_exact_launch(const void* wpack, const float* aux, const float* r
   return launch_exact<exact::IN_NERF>(xp, nerf_xprogram(nullptr), wpack, st);
 }
 
-// raw and d raw / d z at ONE sample per ray on the split-precision kernel: a primal pass that also records the ReLU masks, then
-// the tangent pass t_k = mask_k * (W_k t_{k-1}) over the same packed weights (mlp_exact.cuh, IN_NERF_MASK / IN_NERF_TAN)
-extern "C" size_t b200nerf_nerf_point_jvp_packed_ws_bytes(int n_rays) {
-  return static_cast<size_t>(exact::MAX_STEPS) * static_cast<size_t>(n_rays > 0 ? n_rays : 0) * 4 * sizeof(unsigned long long);
+// raw and d raw / d z at S samples per ray on the split-precision kernel: a primal pass that also records the ReLU masks, then
+// the tangent pass t_k = mask_k * (W_k t_{k-1}) over the same packed weights (mlp_exact.cuh, IN_NERF_MASK / IN_NERF_TAN).
+// Rows are the n_rays * S sample points; row r belongs to ray r / S.
+static size_t jvp_rows(int n_rays, int S) {
+  return n_rays > 0 && S > 0 ? static_cast<size_t>(n_rays) * static_cast<size_t>(S) : 0;
 }
+extern "C" size_t b200nerf_nerf_samples_jvp_packed_ws_bytes(int n_rays, int S) {
+  return static_cast<size_t>(exact::MAX_STEPS) * jvp_rows(n_rays, S) * 4 * sizeof(unsigned long long);
+}
+extern "C" size_t b200nerf_nerf_point_jvp_packed_ws_bytes(int n_rays) { return b200nerf_nerf_samples_jvp_packed_ws_bytes(n_rays, 1); }
+
+// tan_axis < 0: one tangent pass along rays_d (d / dz); 0..2: the pass for unit direction e_axis at explicit pts (d / d pts)
+static int nerf_jvp_packed(const char* who, const void* wpack, const float* aux, const float* rays_o, const float* rays_d,
+                           const float* viewdirs, const float* z, const float* pts, int n_rays, int S, void* ws, float* out_raw,
+                           float* out_tan, cudaStream_t st) {
+  if (n_rays < 0 || S < 1) return fail("%s: bad sizes n_rays=%d S=%d", who, n_rays, S);
+  if (n_rays == 0) return 0;
+  if (jvp_rows(n_rays, S) > 0x7fffffffull) return fail("%s: n_rays * S = %lld sample points exceed 2^31 - 1", who,
+                                                       static_cast<long long>(n_rays) * S);
+  exact::ExactParams xp;
+  memset(&xp, 0, sizeof(xp));
+  xp.aux = aux;
+  xp.n_rows = n_rays * S;
+  xp.S = S;
+  xp.rays_o = rays_o;
+  xp.rays_d = rays_d;
+  xp.viewdirs = viewdirs;
+  xp.z = z;
+  xp.pts = pts;
+  xp.mask = static_cast<unsigned long long*>(ws);
+  xp.head_w_off = NERF_WA;
+  xp.head_b_off = NERF_BA;
+  xp.rgb_w_off = NERF_WR;
+  xp.rgb_b_off = NERF_BR;
+  xp.tan_axis = -1;
+  const XProgram pg = nerf_xprogram(nullptr);
+  xp.out = out_raw;
+  if (launch_exact<exact::IN_NERF_MASK>(xp, pg, wpack, st)) return 1;
+  if (pts == nullptr) {
+    xp.out = out_tan;
+    return launch_exact<exact::IN_NERF_TAN>(xp, pg, wpack, st);
+  }
+  for (int axis = 0; axis < 3; ++axis) {   // out_tan [rows, 3, 4]: the pass for axis k writes slot k of every row
+    xp.tan_axis = axis;
+    xp.out = out_tan + 4 * axis;
+    if (launch_exact<exact::IN_NERF_TAN>(xp, pg, wpack, st)) return 1;
+  }
+  return 0;
+}
+
+extern "C" int b200nerf_nerf_samples_jvp_packed(const void* wpack, const float* aux, const float* rays_o, const float* rays_d,
+                                                const float* viewdirs, const float* z, int n_rays, int S, void* ws, float* out_raw,
+                                                float* out_draw_dz, void* stream) {
+  if (n_rays > 0 && (!wpack || !aux || !rays_o || !rays_d || !viewdirs || !z || !ws || !out_raw || !out_draw_dz))
+    return fail("b200nerf_nerf_samples_jvp_packed: null argument");
+  return nerf_jvp_packed("b200nerf_nerf_samples_jvp_packed", wpack, aux, rays_o, rays_d, viewdirs, z, nullptr, n_rays, S, ws,
+                         out_raw, out_draw_dz, static_cast<cudaStream_t>(stream));
+}
+
 extern "C" int b200nerf_nerf_point_jvp_packed(const void* wpack, const float* aux, const float* rays_o, const float* rays_d,
                                               const float* viewdirs, const float* z, int n_rays, void* ws, float* out_raw,
                                               float* out_draw_dz, void* stream) {
   if (n_rays <= 0) return 0;
   if (!wpack || !aux || !rays_o || !rays_d || !viewdirs || !z || !ws || !out_raw || !out_draw_dz)
     return fail("b200nerf_nerf_point_jvp_packed: null argument");
-  exact::ExactParams xp;
-  memset(&xp, 0, sizeof(xp));
-  xp.aux = aux;
-  xp.n_rows = n_rays;
-  xp.S = 1;
-  xp.rays_o = rays_o;
-  xp.rays_d = rays_d;
-  xp.viewdirs = viewdirs;
-  xp.z = z;
-  xp.mask = static_cast<unsigned long long*>(ws);
-  xp.head_w_off = NERF_WA;
-  xp.head_b_off = NERF_BA;
-  xp.rgb_w_off = NERF_WR;
-  xp.rgb_b_off = NERF_BR;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const XProgram pg = nerf_xprogram(nullptr);
-  xp.out = out_raw;
-  if (launch_exact<exact::IN_NERF_MASK>(xp, pg, wpack, st)) return 1;
-  xp.out = out_draw_dz;
-  return launch_exact<exact::IN_NERF_TAN>(xp, pg, wpack, st);
+  return nerf_jvp_packed("b200nerf_nerf_point_jvp_packed", wpack, aux, rays_o, rays_d, viewdirs, z, nullptr, n_rays, 1, ws, out_raw,
+                         out_draw_dz, static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int b200nerf_nerf_pts_jvp_packed(const void* wpack, const float* aux, const float* pts, const float* viewdirs, int n_rays,
+                                            int S, void* ws, float* out_raw, float* out_draw_dpts, void* stream) {
+  if (n_rays > 0 && (!wpack || !aux || !pts || !viewdirs || !ws || !out_raw || !out_draw_dpts))
+    return fail("b200nerf_nerf_pts_jvp_packed: null argument");
+  return nerf_jvp_packed("b200nerf_nerf_pts_jvp_packed", wpack, aux, nullptr, nullptr, viewdirs, nullptr, pts, n_rays, S, ws, out_raw,
+                         out_draw_dpts, static_cast<cudaStream_t>(stream));
 }
 
 // ------------------------------------------------------------------------------------------- cat-layer chain of the training step

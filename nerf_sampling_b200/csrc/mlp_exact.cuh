@@ -105,6 +105,8 @@ struct ExactParams {
   uint32_t head_w_off, head_b_off;   // sigma head (NeRF) / depth head (DepthNet): 256 weights + bias
   uint32_t rgb_w_off, rgb_b_off;     // rgb head [3,128] + bias
   float radius, near, far;
+  int tan_axis;               // IN_NERF_TAN: < 0 = tangent along rays_d[ray] (d / dz), 0..2 = along the unit axis (d / d pts[axis]);
+                              // an axis pass writes out[row * 3] (the caller offsets out by 4 * axis): out is [rows, 3, 4]
 };
 
 struct __align__(16) Tail {
@@ -616,7 +618,7 @@ __global__ void __launch_bounds__(THREADS, 1) mlp_exact_kernel(const __grid_cons
         if (valid) {
           if (INPUT == IN_NERF_TAN) {
 #pragma unroll
-            for (int t = 0; t < 3; ++t) dir[t] = __ldg(p.rays_d + ray * 3 + t);
+            for (int t = 0; t < 3; ++t) dir[t] = p.tan_axis < 0 ? __ldg(p.rays_d + ray * 3 + t) : (t == p.tan_axis ? 1.f : 0.f);
           }
           if (p.pts != nullptr) {
 #pragma unroll
@@ -813,7 +815,7 @@ __global__ void __launch_bounds__(THREADS, 1) mlp_exact_kernel(const __grid_cons
             named_bar_sync(2 + q, 64);   // the two warps of this lane quarter
             if (TAN) {
               if (sub == 0 && valid)
-                reinterpret_cast<float4*>(p.out)[grow] =
+                reinterpret_cast<float4*>(p.out)[static_cast<size_t>(grow) * (p.tan_axis < 0 ? 1 : 3)] =
                     make_float4(rs + tail->rgb_part[0][row], gs + tail->rgb_part[1][row], bs + tail->rgb_part[2][row],
                                 tail->head_part[0][row] + tail->head_part[1][row] + tail->head_part[2][row] + tail->head_part[3][row]);
             } else if (sub == 0 && valid) {

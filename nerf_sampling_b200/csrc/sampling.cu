@@ -273,3 +273,69 @@ extern "C" int b200nerf_argmax_gather(const float* weights, const float* z, cons
   LAUNCH_CHECK();
   return 0;
 }
+
+// ------------------------------------------------------------------------------------------- placement / points backward
+// sample_points_around_mean (nerf_pytorch/utils.py:220-244) under autograd.  Every placed depth is mean + a constant (the sort only
+// permutes them), so d/d mean is the sum of the S upstream gradients.  Uniform mode clips: torch.clamp passes the gradient where
+// lo <= x <= hi (inclusive) for the UNclipped value x = mean + offset, which is rebuilt here with the forward's rule and rounding
+// (place_uniform_kernel, b200nerf.cu).  One warp per ray.
+__global__ void place_bwd_kernel(const float* __restrict__ mean, const float* __restrict__ grid, int n_rays, int S, int clip, float lo,
+                                 float hi, const float* __restrict__ g_z, float* __restrict__ g_mean) {
+  const int ray = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  const int lane = threadIdx.x & 31;
+  if (ray >= n_rays) return;
+  const float m = clip ? __ldg(mean + ray) : 0.f;
+  float acc = 0.f;
+  for (int s = lane; s < S; s += 32) {
+    const float g = __ldg(g_z + static_cast<size_t>(ray) * S + s);
+    if (clip) {
+      float x = m;
+      if (s <= S - 2 && __ldg(grid + s) < 0.f) x = __fadd_rn(m, __ldg(grid + s));
+      else if (s >= 1 && !(__ldg(grid + s - 1) < 0.f)) x = __fadd_rn(m, __ldg(grid + s - 1));
+      if (!(x >= lo && x <= hi)) continue;
+    }
+    acc += g;
+  }
+#pragma unroll
+  for (int off = 16; off > 0; off >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, off);
+  if (lane == 0) g_mean[ray] = acc;
+}
+
+extern "C" int b200nerf_place_samples_bwd(const float* mean, const float* offsets, int n_rays, int S, int mode, float clip_lo,
+                                          float clip_hi, const float* g_z, float* out_g_mean, void* stream) {
+  if (n_rays < 0 || S < 1) return b200_fail("b200nerf_place_samples_bwd: bad sizes n_rays=%d S=%d", n_rays, S);
+  if (mode != B200NERF_PLACE_DEPTH_ONLY && mode != B200NERF_PLACE_UNIFORM && mode != B200NERF_PLACE_GAUSSIAN)
+    return b200_fail("b200nerf_place_samples_bwd: unknown mode %d", mode);
+  if (mode == B200NERF_PLACE_DEPTH_ONLY && S != 1) return b200_fail("b200nerf_place_samples_bwd: depth_only needs S == 1");
+  if (n_rays == 0) return 0;
+  if (!mean || !g_z || !out_g_mean) return b200_fail("b200nerf_place_samples_bwd: null argument");
+  const bool clip = mode == B200NERF_PLACE_UNIFORM;
+  if (clip && S > 1 && !offsets) return b200_fail("b200nerf_place_samples_bwd: offsets is null (uniform mode needs the grid)");
+  const int wpb = 8;
+  place_bwd_kernel<<<(n_rays + wpb - 1) / wpb, wpb * 32, 0, static_cast<cudaStream_t>(stream)>>>(mean, offsets, n_rays, S, clip ? 1 : 0,
+                                                                                             clip_lo, clip_hi, g_z, out_g_mean);
+  LAUNCH_CHECK();
+  return 0;
+}
+
+// pts = rays_o + rays_d z (b200nerf_points) backward: g_z = sum_k g_pts[k] rays_d[k]
+__global__ void points_bwd_kernel(const float* __restrict__ rd, const float* __restrict__ g_pts, size_t total, int S,
+                                  float* __restrict__ g_z) {
+  const size_t i = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (i >= total) return;
+  const size_t ray = i / S;
+  const float* g = g_pts + i * 3;
+  g_z[i] = __fadd_rn(__fadd_rn(__fmul_rn(__ldg(g), __ldg(rd + ray * 3)), __fmul_rn(__ldg(g + 1), __ldg(rd + ray * 3 + 1))),
+                     __fmul_rn(__ldg(g + 2), __ldg(rd + ray * 3 + 2)));
+}
+
+extern "C" int b200nerf_points_bwd(const float* rays_d, const float* g_pts, int n_rays, int S, float* out_g_z, void* stream) {
+  if (n_rays < 0 || S < 1) return b200_fail("b200nerf_points_bwd: bad sizes n_rays=%d S=%d", n_rays, S);
+  const size_t total = static_cast<size_t>(n_rays) * S;
+  if (total == 0) return 0;
+  if (!rays_d || !g_pts || !out_g_z) return b200_fail("b200nerf_points_bwd: null argument");
+  points_bwd_kernel<<<static_cast<unsigned>((total + 255) / 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(rays_d, g_pts, total, S,
+                                                                                                          out_g_z);
+  LAUNCH_CHECK();
+  return 0;
+}

@@ -1479,19 +1479,21 @@ extern "C" int b200nerf_depthnet_train_bwd_jac(const float* const* params, int n
                                                   stream_aux);
 }
 
-// ------------------------------------------------------------------------------------------- NeRF at one sample per ray + d/dz
+// ------------------------------------------------------------------------------------------- NeRF at S samples per ray + d/dz
 // rows 0..n-1 = primal gamma(p), rows n..2n-1 = tangent d gamma(p) / dz, p = o + d z, row width d = 3 (1 + 2 nf); view encoding
-// [n, dv], dv = 3 (1 + 2 nv).  Six threads per ray: three position channels (nf sincosf each) and three view-direction channels (nv).
+// [n, dv], dv = 3 (1 + 2 nv).  n = n_rays * S rows; row i belongs to ray i / S.  Six threads per row: three position channels
+// (nf sincosf each) and three view-direction channels (nv).
 __global__ void nerf_point_encode_kernel(const float* __restrict__ ro, const float* __restrict__ rd, const float* __restrict__ vd,
-                                         const float* __restrict__ z, int n, int nf, int nv, float* __restrict__ enc,
+                                         const float* __restrict__ z, int n, int S, int nf, int nv, float* __restrict__ enc,
                                          float* __restrict__ venc) {
-  const int t = blockIdx.x * blockDim.x + threadIdx.x;
-  const int i = t / 6, c = t % 3;
+  const long long t = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+  const int i = static_cast<int>(t / 6), c = static_cast<int>(t % 3);
   if (i >= n) return;
+  const size_t ray = static_cast<size_t>(i / S);
   if (t % 6 < 3) {
     const int d3 = 3 * (1 + 2 * nf);
-    const float d = rd[i * 3 + c];
-    const float x = __fadd_rn(ro[i * 3 + c], __fmul_rn(d, z[i]));
+    const float d = rd[ray * 3 + c];
+    const float x = __fadd_rn(ro[ray * 3 + c], __fmul_rn(d, z[i]));
     float* p = enc + static_cast<size_t>(i) * d3;
     float* tg = enc + static_cast<size_t>(n + i) * d3;
     p[c] = x;
@@ -1506,7 +1508,7 @@ __global__ void nerf_point_encode_kernel(const float* __restrict__ ro, const flo
       tg[3 + j * 6 + 3 + c] = -f * s * d;
     }
   } else {
-    const float v = vd[i * 3 + c];
+    const float v = vd[ray * 3 + c];
     float* e = venc + static_cast<size_t>(i) * (3 * (1 + 2 * nv));
     e[c] = v;
     for (int j = 0; j < nv; ++j) {
@@ -1584,30 +1586,41 @@ static bool nerf_point_multires_ok(int multires, int multires_views) {
   return multires >= 1 && multires <= 10 && multires_views >= 1 && multires_views <= 4;
 }
 // the layout holds the widest encodings (d <= 64, dv <= 32), so the size does not depend on multires / multires_views
-extern "C" size_t b200nerf_nerf_point_ws_floats_multires(int n_rays, int multires, int multires_views) {
+extern "C" size_t b200nerf_nerf_samples_ws_floats_multires(int n_rays, int S, int multires, int multires_views) {
   if (!nerf_point_multires_ok(multires, multires_views)) {
     b200_fail("b200nerf_nerf_point_ws_floats: multires=%d / multires_views=%d out of range (multires 1..10, multires_views 1..4)",
               multires, multires_views);
     return 0;
   }
-  const size_t n = static_cast<size_t>(n_rays);
+  if (n_rays < 0 || S < 1) {
+    b200_fail("b200nerf_nerf_samples_ws_floats: bad sizes n_rays=%d S=%d", n_rays, S);
+    return 0;
+  }
+  const size_t n = static_cast<size_t>(n_rays) * static_cast<size_t>(S);
   return 2 * n * 64 + n * 32 + 3 * (2 * n * 256) + 2 * n * 4 + 2 * n + 256;
+}
+extern "C" size_t b200nerf_nerf_point_ws_floats_multires(int n_rays, int multires, int multires_views) {
+  return b200nerf_nerf_samples_ws_floats_multires(n_rays, 1, multires, multires_views);
 }
 extern "C" size_t b200nerf_nerf_point_ws_floats(int n_rays) { return b200nerf_nerf_point_ws_floats_multires(n_rays, 10, 4); }
 
 // params: the 24 fp32 device tensors of NeRF in state_dict order (see b200nerf_nerf_pack) at multires / multires_views:
 // pts_linears.0 is [256, d], pts_linears.5 [256, d + 256], views_linears.0 [128, 256 + dv]
-extern "C" int b200nerf_nerf_point_jvp_multires(const float* const* t, int multires, int multires_views, const float* rays_o,
-                                                const float* rays_d, const float* viewdirs, const float* z, int n_rays, float* ws,
-                                                float* out_raw, float* out_draw_dz, void* stream) {
+// S samples per ray: z [n_rays, S], out_raw / out_draw_dz [n_rays * S, 4]; every product runs over the n_rays * S rows
+extern "C" int b200nerf_nerf_samples_jvp_multires(const float* const* t, int multires, int multires_views, const float* rays_o,
+                                                  const float* rays_d, const float* viewdirs, const float* z, int n_rays, int S,
+                                                  float* ws, float* out_raw, float* out_draw_dz, void* stream) {
   if (!nerf_point_multires_ok(multires, multires_views))
     return b200_fail("b200nerf_nerf_point_jvp: multires=%d / multires_views=%d out of range (multires 1..10, multires_views 1..4)",
                      multires, multires_views);
+  if (S < 1) return b200_fail("b200nerf_nerf_samples_jvp: S=%d; S >= 1 is required", S);
   if (n_rays <= 0) return 0;
+  if (static_cast<long long>(n_rays) * S > (1ll << 26))   // 2^26 rows need ~460 GB of workspace; the row indices stay in int
+    return b200_fail("b200nerf_nerf_samples_jvp: n_rays * S = %lld rows exceed 2^26", static_cast<long long>(n_rays) * S);
   if (!t || !rays_o || !rays_d || !viewdirs || !z || !ws || !out_raw || !out_draw_dz) return b200_fail("b200nerf_nerf_point_jvp: null argument");
   const int d = 3 * (1 + 2 * multires), dv = 3 * (1 + 2 * multires_views), ld5 = 256 + d, ldv = 256 + dv;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const int n = n_rays, n2 = 2 * n_rays;
+  const int n = n_rays * S, n2 = 2 * n;
   float* enc = ws;                                   // [2n, d]
   float* venc = enc + static_cast<size_t>(n2) * 64;  // [n, dv]
   float* h0 = venc + static_cast<size_t>(n) * 32;    // [2n, 256]
@@ -1615,7 +1628,8 @@ extern "C" int b200nerf_nerf_point_jvp_multires(const float* const* t, int multi
   float* h2 = h1 + static_cast<size_t>(n2) * 256;
   float* rgb2 = h2 + static_cast<size_t>(n2) * 256;  // [2n, 3]
   float* al2 = rgb2 + static_cast<size_t>(n2) * 4;   // [2n]
-  nerf_point_encode_kernel<<<(6 * n + 191) / 192, 192, 0, st>>>(rays_o, rays_d, viewdirs, z, n, multires, multires_views, enc, venc);
+  nerf_point_encode_kernel<<<static_cast<unsigned>((6ll * n + 191) / 192), 192, 0, st>>>(rays_o, rays_d, viewdirs, z, n, S, multires,
+                                                                                         multires_views, enc, venc);
   LAUNCH_CHECK();
   auto act = [&](float* Y, const float* bias, int M, int relu) -> int {
     const size_t tot = static_cast<size_t>(n) * M;
@@ -1731,6 +1745,13 @@ extern "C" int b200nerf_nerf_point_jvp_multires(const float* const* t, int multi
   nerf_point_out_kernel<<<(n + 255) / 256, 256, 0, st>>>(rgb2, al2, t[23], t[21], n, out_raw, out_draw_dz);
   LAUNCH_CHECK();
   return 0;
+}
+
+extern "C" int b200nerf_nerf_point_jvp_multires(const float* const* t, int multires, int multires_views, const float* rays_o,
+                                                const float* rays_d, const float* viewdirs, const float* z, int n_rays, float* ws,
+                                                float* out_raw, float* out_draw_dz, void* stream) {
+  return b200nerf_nerf_samples_jvp_multires(t, multires, multires_views, rays_o, rays_d, viewdirs, z, n_rays, 1, ws, out_raw,
+                                            out_draw_dz, stream);
 }
 
 extern "C" int b200nerf_nerf_point_jvp(const float* const* t, const float* rays_o, const float* rays_d, const float* viewdirs,

@@ -103,16 +103,18 @@ class NeRF(nn.Module):
         return self._packed
 
     def query(self, viewdirs, *, rays_o=None, rays_d=None, z=None, pts=None):
-        """raw [N,S,4] for sample positions o + d*z (or explicit pts) with fused encodings.  When ``z`` carries a
-        gradient (training: one DepthNet sample per ray through the frozen NeRF, nerf_utils.py:692-715) the
-        forward-mode route evaluates raw and d raw / d z (training.NerfPointFn)."""
-        if z is not None and z.requires_grad and torch.is_grad_enabled():
-            if z.shape[-1] != 1:
-                raise NotImplementedError("gradients w.r.t. sample depths are implemented for one sample per ray")
+        """raw [N,S,4] for sample positions o + d*z (or explicit pts) with fused encodings.  When ``z`` or ``pts``
+        carries a gradient (the training render through the frozen NeRF, nerf_utils.py:692-715, or a user objective
+        through the S-sample render) the forward-mode route evaluates raw at split precision together with d raw / d z
+        (training.NerfPointFn) or d raw / d pts (training.NerfPtsFn).  The NeRF's own parameters get no gradient."""
+        if torch.is_grad_enabled():
             from .. import training
 
-            return training.NerfPointFn.apply(z, rays_o.contiguous().float(), rays_d.contiguous().float(),
-                                              viewdirs.contiguous().float(), self.packed(), *training.nerf_params(self))
+            if z is not None and z.requires_grad:
+                return training.NerfPointFn.apply(z, rays_o.contiguous().float(), rays_d.contiguous().float(),
+                                                  viewdirs.contiguous().float(), self.packed(), *training.nerf_params(self))
+            if z is None and pts is not None and pts.requires_grad:
+                return training.NerfPtsFn.apply(pts, viewdirs, self.packed())
         return ops.nerf_mlp(self.packed(), viewdirs, rays_o=rays_o, rays_d=rays_d, z=z, pts=pts)
 
     def forward(self, x):

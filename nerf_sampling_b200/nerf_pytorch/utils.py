@@ -99,6 +99,12 @@ def sample_points_around_mean(rays_o, rays_d, mean, n_samples=32, mode="gaussian
     """(pts [N,S,3], z_vals [N,S]) around the predicted depth (utils.py:220-244).
 
     ``noise`` ([N, n_samples-1] standard normal) makes gaussian mode reproducible; by default it is drawn with
-    ``torch.randn`` like the reference."""
+    ``torch.randn`` like the reference.  When grad is enabled and ``mean`` requires it, z and pts are differentiable
+    w.r.t. ``mean`` (training.PlaceFn / training.PointsFn; the rays get no gradient)."""
+    if torch.is_grad_enabled() and isinstance(mean, torch.Tensor) and mean.requires_grad:
+        from .. import training
+
+        z = training.PlaceFn.apply(mean, n_samples, mode, std, noise)
+        return training.PointsFn.apply(rays_o, rays_d, z), z
     z = ops.place_samples(mean, n_samples, mode, std, noise)
     return ops.points(rays_o, rays_d, z), z

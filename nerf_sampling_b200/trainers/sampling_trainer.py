@@ -64,9 +64,21 @@ class DepthNetTrainer(Blender.BlenderTrainer):
         """(rgb_map, disp_map, acc_map, depth_map, density, alphas, weights) -- sampling_trainer.py:153-230.
 
         Unknown keyword arguments are swallowed exactly like the reference's ``**kwargs`` (its DepthNet call sites pass
-        misspelled ``raw_noise=`` / ``white_bkdg=``, which is why that path always composites noise-free on white)."""
+        misspelled ``raw_noise=`` / ``white_bkdg=``, which is why that path always composites noise-free on white).
+
+        When grad is enabled and ``raw`` or ``z_vals`` requires it, the maps are differentiable w.r.t. both
+        (training.CompositeFn; at S == 1 training.CompositeSingleFn, whose only dependence is rgb on raw)."""
         noise = None
         if raw_noise_std > 0.0:
             noise = torch.randn(raw[..., 3].shape, device=raw.device) * raw_noise_std
+        if torch.is_grad_enabled() and (raw.requires_grad or z_vals.requires_grad):
+            from .. import training
+
+            if z_vals.shape[-1] >= 2:
+                rgb, disp, acc, depth, weights, alphas = training.CompositeFn.apply(raw, z_vals, rays_d, noise, white_bkgd)
+            else:
+                rgb, disp = training.CompositeSingleFn.apply(raw, z_vals, rays_d)
+                _, _, acc, depth, weights, alphas = ops.composite(raw.detach(), z_vals.detach(), rays_d, white_bkgd, noise)
+            return rgb, disp, acc, depth, raw[..., 3], alphas, weights
         rgb, disp, acc, depth, weights, alphas = ops.composite(raw, z_vals, rays_d, white_bkgd, noise)
         return rgb, disp, acc, depth, raw[..., 3], alphas, weights

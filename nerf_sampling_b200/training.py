@@ -101,38 +101,41 @@ class DepthNetTrainFn(torch.autograd.Function):
 JVP_MODE = __import__("os").environ.get("B200NERF_TRAIN_JVP", "split")
 
 
-def nerf_point_jvp(packed, params, rays_o, rays_d, viewdirs, z_flat, raw, draw, stream):
-    """Fills raw [n,1,4] and draw [n,4]; ``packed`` (a packing.PackedNeRF with a split-precision stream) selects the packed route.
-    Returns the workspace tensor, which must stay alive until the launches have run."""
+def nerf_point_jvp(packed, params, rays_o, rays_d, viewdirs, z_flat, raw, draw, stream, S=1):
+    """Fills raw [n*S,...,4] and draw [n*S,4] at the sample depths z_flat (n*S values, ray-major: sample r belongs to ray r // S);
+    ``packed`` (a packing.PackedNeRF with a split-precision stream) selects the packed route.  Returns the workspace tensor, which
+    must stay alive until the launches have run."""
     L = _lib.lib()
-    n, dev = z_flat.shape[0], z_flat.device
+    n, dev = z_flat.shape[0] // S, z_flat.device
     if packed is not None and packed.wpack is not None and JVP_MODE == "split":
-        ws = torch.empty(L.b200nerf_nerf_point_jvp_packed_ws_bytes(n), dtype=torch.uint8, device=dev)
-        _lib.check(L.b200nerf_nerf_point_jvp_packed(packed.wpack.data_ptr(), packed.aux.data_ptr(), rays_o.data_ptr(), rays_d.data_ptr(),
-                                                    viewdirs.data_ptr(), z_flat.data_ptr(), n, ws.data_ptr(), raw.data_ptr(),
-                                                    draw.data_ptr(), stream))
+        ws = torch.empty(L.b200nerf_nerf_samples_jvp_packed_ws_bytes(n, S), dtype=torch.uint8, device=dev)
+        _lib.check(L.b200nerf_nerf_samples_jvp_packed(packed.wpack.data_ptr(), packed.aux.data_ptr(), rays_o.data_ptr(),
+                                                      rays_d.data_ptr(), viewdirs.data_ptr(), z_flat.data_ptr(), n, S, ws.data_ptr(),
+                                                      raw.data_ptr(), draw.data_ptr(), stream))
         return ws
     # the packed route reads the encodings' sizes from its aux block; this one takes them from the tensors' shapes
     mr = packing.nerf_multires(dict(zip(packing.NERF_KEYS, params)))
-    ws = torch.empty(L.b200nerf_nerf_point_ws_floats_multires(n, *mr), device=dev)
-    _lib.check(L.b200nerf_nerf_point_jvp_multires(_ptrs(list(params)), *mr, rays_o.data_ptr(), rays_d.data_ptr(), viewdirs.data_ptr(),
-                                                  z_flat.data_ptr(), n, ws.data_ptr(), raw.data_ptr(), draw.data_ptr(), stream))
+    ws = torch.empty(L.b200nerf_nerf_samples_ws_floats_multires(n, S, *mr), device=dev)
+    _lib.check(L.b200nerf_nerf_samples_jvp_multires(_ptrs(list(params)), *mr, rays_o.data_ptr(), rays_d.data_ptr(), viewdirs.data_ptr(),
+                                                    z_flat.data_ptr(), n, S, ws.data_ptr(), raw.data_ptr(), draw.data_ptr(), stream))
     return ws
 
 
 class NerfPointFn(torch.autograd.Function):
-    """raw [N,1,4] of the frozen NeRF at p = o + d z (one sample per ray), differentiable w.r.t. z.  ``packed``: the model's
-    packing.PackedNeRF (split-precision route, see JVP_MODE) or None (fp32 route over ``params``)."""
+    """raw [N,S,4] of the frozen NeRF at p = o + d z for z [N,S] (or [N]: one sample per ray), differentiable w.r.t. z through
+    the forward-mode d raw / d z.  ``packed``: the model's packing.PackedNeRF (split-precision route, see JVP_MODE) or None
+    (fp32 route over ``params``)."""
 
     @staticmethod
     def forward(ctx, z, rays_o, rays_d, viewdirs, packed, *params):
         n = z.shape[0]
+        S = z.shape[1] if z.dim() > 1 else 1
         dev = z.device
-        raw = torch.empty(n, 1, 4, device=dev)
-        draw = torch.empty(n, 4, device=dev)
+        raw = torch.empty(n, S, 4, device=dev)
+        draw = torch.empty(n * S, 4, device=dev)
         zz = z.detach().reshape(-1).contiguous().float()
         with torch.cuda.device(dev):
-            nerf_point_jvp(packed, params, rays_o, rays_d, viewdirs, zz, raw, draw, _stream())
+            nerf_point_jvp(packed, params, rays_o, rays_d, viewdirs, zz, raw, draw, _stream(), S=S)
         ctx.save_for_backward(draw)
         ctx.zshape = z.shape
         return raw
@@ -142,6 +145,39 @@ class NerfPointFn(torch.autograd.Function):
         (draw,) = ctx.saved_tensors
         gz = (g_raw.reshape(-1, 4) * draw).sum(-1).reshape(ctx.zshape)  # chain rule over the four outputs
         return (gz, None, None, None, None) + (None,) * 24
+
+
+class NerfPtsFn(torch.autograd.Function):
+    """raw [N,S,4] of the frozen NeRF at explicit points pts [N,S,3] (Trainer.run_network), differentiable w.r.t. pts through the
+    Jacobian d raw / d pts [N*S,3,4] of the split-precision kernel (b200nerf_nerf_pts_jvp_packed)."""
+
+    @staticmethod
+    def forward(ctx, pts, viewdirs, packed):
+        if packed.wpack is None:
+            raise _lib.B200NerfError(
+                f"gradients w.r.t. sample points need the split-precision weight image; this NeRF is packed at precision "
+                f"{packed.prec} (PREC_FP16 = {packing.PREC_FP16} has none): use PREC_SPLIT or PREC_FAST")
+        from . import ops
+
+        L = _lib.lib()
+        n, S = pts.shape[0], pts.shape[1]
+        p, viewdirs = ops._dev(pts.detach(), "pts"), ops._dev(viewdirs, "viewdirs")
+        dev = p.device
+        raw = torch.empty(n, S, 4, device=dev)
+        jac = torch.empty(n * S, 3, 4, device=dev)
+        ws = torch.empty(L.b200nerf_nerf_samples_jvp_packed_ws_bytes(n, S), dtype=torch.uint8, device=dev)
+        with torch.cuda.device(dev):
+            _lib.check(L.b200nerf_nerf_pts_jvp_packed(packed.wpack.data_ptr(), packed.aux.data_ptr(), p.data_ptr(), viewdirs.data_ptr(),
+                                                      n, S, ws.data_ptr(), raw.data_ptr(), jac.data_ptr(), _stream()))
+        ctx.save_for_backward(jac)
+        ctx.pshape = pts.shape
+        return raw
+
+    @staticmethod
+    def backward(ctx, g_raw):
+        (jac,) = ctx.saved_tensors
+        g = (g_raw.reshape(-1, 1, 4) * jac).sum(-1)   # sum over the four outputs of d raw_c / d pts_k
+        return g.reshape(ctx.pshape), None, None
 
 
 class CompositeSingleFn(torch.autograd.Function):
@@ -162,6 +198,91 @@ class CompositeSingleFn(torch.autograd.Function):
         g = torch.zeros(rgb.shape[0], 1, 4, device=rgb.device)
         g[:, 0, :3] = g_rgb * rgb * (1.0 - rgb)
         return g, None, None
+
+
+class CompositeFn(torch.autograd.Function):
+    """raw2outputs for S >= 2 (trainers/sampling_trainer.py:153-230) -> (rgb, disp, acc, depth, weights, alphas), differentiable
+    w.r.t. raw and z through b200nerf_composite_bwd.  ``noise`` [N,S] (already scaled) or None is the draw the forward used."""
+
+    @staticmethod
+    def forward(ctx, raw, z, rays_d, noise, white_bkgd):
+        from . import ops
+
+        ctx.set_materialize_grads(False)
+        outs = ops.composite(raw.detach(), z.detach(), rays_d, white_bkgd, noise)
+        ctx.save_for_backward(raw, z, rays_d, noise)
+        ctx.white = bool(white_bkgd)
+        return outs
+
+    @staticmethod
+    def backward(ctx, g_rgb, g_disp, g_acc, g_depth, g_weights, g_alphas):
+        raw, z, rays_d, noise = ctx.saved_tensors
+        L = _lib.lib()
+        n, S = z.shape
+        dev = raw.device
+        f = lambda t: None if t is None else t.detach().contiguous().float()  # noqa: E731
+        raw_c, z_c, rd, nz = f(raw), f(z), f(rays_d), f(noise)
+        gs = [f(g) for g in (g_rgb, g_disp, g_acc, g_depth, g_weights, g_alphas)]
+        g_raw = torch.empty(n, S, 4, device=dev)
+        g_z = torch.empty(n, S, device=dev)
+        p = lambda t: None if t is None else t.data_ptr()  # noqa: E731
+        with torch.cuda.device(dev):
+            _lib.check(L.b200nerf_composite_bwd(raw_c.data_ptr(), z_c.data_ptr(), rd.data_ptr(), p(nz), n, S, int(ctx.white),
+                                                *[p(g) for g in gs], g_raw.data_ptr(), g_z.data_ptr(), _stream()))
+        return (g_raw.reshape(raw.shape) if ctx.needs_input_grad[0] else None,
+                g_z if ctx.needs_input_grad[1] else None, None, None, None)
+
+
+class PlaceFn(torch.autograd.Function):
+    """z [N,S] of sample_points_around_mean (ops.place_samples), differentiable w.r.t. ``mean`` (b200nerf_place_samples_bwd)."""
+
+    @staticmethod
+    def forward(ctx, mean, n_samples, mode, std, noise):
+        from . import ops
+
+        z = ops.place_samples(mean.detach(), n_samples, mode, std, noise)
+        ctx.save_for_backward(mean)
+        ctx.cfg = (z.shape[1], mode, float(std))
+        return z
+
+    @staticmethod
+    def backward(ctx, g_z):
+        from . import ops
+
+        (mean,) = ctx.saved_tensors
+        S, mode, std = ctx.cfg
+        m = mean.detach().reshape(-1).contiguous().float()
+        n = m.shape[0]
+        grid = ops.uniform_grid(std, S, m.device) if (mode == "uniform" and S > 1) else None
+        g = g_z.contiguous().float()
+        g_mean = torch.empty(n, device=m.device)
+        with torch.cuda.device(m.device):
+            _lib.check(_lib.lib().b200nerf_place_samples_bwd(m.data_ptr(), None if grid is None else grid.data_ptr(), n, S,
+                                                             ops.PLACE_MODES[mode], 2.0, 6.0, g.data_ptr(), g_mean.data_ptr(),
+                                                             _stream()))
+        return g_mean.reshape(mean.shape), None, None, None, None
+
+
+class PointsFn(torch.autograd.Function):
+    """pts [N,S,3] = o + d z (ops.points), differentiable w.r.t. z (b200nerf_points_bwd); rays get no gradient."""
+
+    @staticmethod
+    def forward(ctx, rays_o, rays_d, z):
+        from . import ops
+
+        rd = rays_d.detach().contiguous().float()
+        ctx.save_for_backward(rd)
+        return ops.points(rays_o.detach(), rd, z.detach())
+
+    @staticmethod
+    def backward(ctx, g_pts):
+        (rd,) = ctx.saved_tensors
+        n, S = g_pts.shape[0], g_pts.shape[1]
+        g = g_pts.contiguous().float()
+        g_z = torch.empty(n, S, device=g.device)
+        with torch.cuda.device(g.device):
+            _lib.check(_lib.lib().b200nerf_points_bwd(rd.data_ptr(), g.data_ptr(), n, S, g_z.data_ptr(), _stream()))
+        return None, None, g_z
 
 
 def nerf_params(module) -> List[torch.nn.Parameter]:
